@@ -65,6 +65,11 @@ def parse():
     ap.add_argument("--host-obs-dtype", default=None, choices=[None, "float32", "float16"],
                     help="e2e leg: dtype of the observations on the host (default: float32, the reference's Box dtype)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed env.step returned (rank 0) as DIR/<name>.npy "
+                         "in float32 / float64, at most 64 MB in all: above that, every array keeps the rows "
+                         "sorted(np.random.default_rng(0).permutation(n)[:k]) of its n environments, k = n x budget "
+                         "share; bool and integer outputs are stored as float32 / float64")
     return ap.parse_args()
 
 
@@ -259,8 +264,10 @@ def gpu_arm(args):
     env.reset(seed=1234)
 
     # ---- device-resident throughput ("value") ------------------------------------------
+    last = [None]
+
     def dev_step(i):
-        env.step(pool[i % len(pool)])
+        last[0] = env.step(pool[i % len(pool)])
 
     for i in range(args.warmup):
         dev_step(i)
@@ -279,6 +286,9 @@ def gpu_arm(args):
     stats = env.episode_statistics(reduce=True)
     member_stats = stats.get("members", [stats])
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # copy_outputs=False: the returned tensors alias engine buffers that the e2e leg below overwrites
+        dump_outputs(args.dump_outputs, last[0])
 
     # ---- end to end through the public API with HOST buffers ("e2e") ---------------------
     # env.step_host: actions from a pinned host buffer, results (next observation, reward, cost,
@@ -410,6 +420,49 @@ def csrc_hash():
     for name in ("opfg_core.h", "opfg_api.cu", "symbolic.cpp", "symbolic.hpp"):
         h.update(open(os.path.join(ROOT, "opfgym_b200", "csrc", name), "rb").read())
     return h.hexdigest()
+
+
+DUMP_BUDGET = 60 << 20          # bytes of array data: with the .npy headers, under 64 MB
+
+
+def dump_outputs(out_dir, result):
+    """Write the tensors of one ``env.step`` result ``(obs, reward, terminated, truncated, info)`` -- nested
+    info entries (a mixed batch's ``member`` list) included -- as ``out_dir/<name>.npy``."""
+    import numpy as np
+    import torch
+
+    arrays = {}
+
+    def walk(name, x):
+        if isinstance(x, torch.Tensor):
+            arrays[name] = x
+        elif isinstance(x, dict):
+            for k, v in x.items():
+                walk(f"{name}_{k}", v)
+        elif isinstance(x, (list, tuple)):
+            for k, v in enumerate(x):
+                walk(f"{name}_{k}", v)
+
+    for name, x in zip(("obs", "reward", "terminated", "truncated", "info"), result):
+        walk(name, x)
+
+    def as_float(t):
+        if t.dtype in (torch.float32, torch.float64):
+            return t
+        if t.is_floating_point() or t.dtype == torch.bool or t.element_size() <= 2:
+            return t.to(torch.float32)
+        return t.to(torch.float64)
+
+    arrays = {k: as_float(v.detach()) for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in arrays.values())
+    share = min(1.0, DUMP_BUDGET / max(total, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if share < 1.0 and t.dim() > 0:
+            n = t.shape[0]
+            rows = np.sort(np.random.default_rng(0).permutation(n)[:max(1, int(n * share))])
+            t = t.index_select(0, torch.as_tensor(rows, device=t.device))
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 def single_env_row(kind, dev, n=200):

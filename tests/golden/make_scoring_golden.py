@@ -1,8 +1,10 @@
 #!/usr/bin/env python
-"""Generate tests/golden/scoring_cases.npz: outputs of the reference's OWN
+"""Generate tests/golden/scoring_cases.npz.xz: outputs of the reference's OWN
 ``opfgym/objective.py``, ``opfgym/constraints.py`` and ``opfgym/reward.py``
 (imported unmodified from /root/reference, pandapower stubbed for the type hint
 only) on random result tables.  Run from the repo root in the build container."""
+import io
+import lzma
 import os
 import sys
 
@@ -107,8 +109,13 @@ def main():
         arrays[f"case{k}/reward"] = np.array(float(rf(objective, penalty, valid)))
         arrays[f"case{k}/cost"] = np.array(float(rf.calculate_cost(penalty, valid)))
         arrays[f"case{k}/constraint_names"] = np.array([type(c).__name__ for c in cons])
-    path = os.path.join(HERE, "scoring_cases.npz")
-    np.savez_compressed(path, **arrays)
+    # an uncompressed npz under one xz stream: the ~5 000 small members share one dictionary, and their zip
+    # headers and names compress away
+    path = os.path.join(HERE, "scoring_cases.npz.xz")
+    buf = io.BytesIO()
+    np.savez(buf, **arrays)
+    with lzma.open(path, "wb", preset=9 | lzma.PRESET_EXTREME) as f:
+        f.write(buf.getvalue())
     print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 

@@ -1,4 +1,4 @@
-"""(De)serialisation of the small random nets of tests/golden/scoring_cases.npz and
+"""(De)serialisation of the small random nets of tests/golden/scoring_cases.npz.xz and
 the parameter sets cycled through by its generator."""
 import numpy as np
 import pandas as pd

@@ -3,6 +3,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -30,7 +32,13 @@ def test_cuda_library_exports_every_symbol():
         assert getattr(lib, name) is not None
     capi.declare(lib)
     assert lib.opfg_version() == 1
-    assert lib.opfg_launch_count() == 0
+    # the launch counter of a freshly loaded library starts at 0: checked in a new process, because earlier
+    # tests of this session may have launched kernels through the same (process-wide) library
+    code = ("import ctypes, sys; lib = ctypes.CDLL(sys.argv[1]); lib.opfg_launch_count.restype = ctypes.c_int64; "
+            "print(lib.opfg_launch_count())")
+    res = subprocess.run([sys.executable, "-c", code, capi.LIB_PATH], capture_output=True, text=True, timeout=300)
+    assert res.returncode == 0, res.stderr[-2000:]
+    assert int(res.stdout) == 0
 
 
 def test_no_cpu_fallback_in_product():

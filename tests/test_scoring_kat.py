@@ -2,6 +2,9 @@
 tests/test_constraints.py, tests/test_objective.py, tests/test_reward.py), replayed on
 (a) the CPU oracle (oracle/scoring.py) and (b) the product's scalar host mirror; plus
 the randomised fixture produced by the reference's own modules."""
+import io
+import lzma
+
 import numpy as np
 import pandas as pd
 import pytest
@@ -201,7 +204,8 @@ def test_reward_known_answers(call):        # reference tests/test_reward.py:8-7
 
 # -------------------------------------------- randomised cases from the reference modules
 def _cases():
-    z = np.load(gs.__file__.replace("golden_scoring_util.py", "golden/scoring_cases.npz"))
+    with lzma.open(gs.__file__.replace("golden_scoring_util.py", "golden/scoring_cases.npz.xz")) as f:
+        z = np.load(io.BytesIO(f.read()))
     return z, int(z["n_cases"])
 
 
