@@ -107,6 +107,10 @@ typedef struct {
     int32_t radial_lanes_per_env, radial_envs_per_cta, radial_smem_bytes_per_env;
     int32_t n_island_critical; /* dynamic branches whose outage can cut buses off (spanning-tree edges): only then
                                   does opfg_assemble walk the grid of an environment                     */
+    int32_t cta_envs_per_cta;  /* CTA kernel: environments per CTA (1 = k_pf, one CTA per environment; > 1 = k_pf_multi) */
+    int32_t cta_tables_staged; /* k_pf_multi: tables staged in shared memory, 0 = LU schedule + Ybus index tables,
+                                  1 = + Ybus values, 2 = + start-value / DC / q-limit tables                  */
+    int32_t score_threads_per_env; /* opfg_score: threads per environment (32 = k_score_warps, else k_score) */
 } OpfgGridInfo;
 
 /* action application + Sbus scatter (kernel 1) */

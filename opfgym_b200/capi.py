@@ -39,7 +39,8 @@ class GridInfo(C.Structure):
                [(n, C.c_int32) for n in ("pf_kernel_used", "lane_max_row", "lane_warps_per_cta",
                                          "lane_tables_staged")] + [("lane_scratch_bytes", C.c_double)] + \
                [(n, C.c_int32) for n in ("radial_lanes_per_env", "radial_envs_per_cta",
-                                         "radial_smem_bytes_per_env", "n_island_critical")]
+                                         "radial_smem_bytes_per_env", "n_island_critical",
+                                         "cta_envs_per_cta", "cta_tables_staged", "score_threads_per_env")]
 
 
 class AssemblyDesc(C.Structure):

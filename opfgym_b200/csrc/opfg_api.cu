@@ -127,6 +127,7 @@ struct OpfgGrid {
     int n_blocks_sym = 0;          // blocks of the filled Jacobian (d.n_blocks counts storage slots)
     int carveout_pct = -1;   // -1: leave the driver's default L1/shared split
     int envs_per_cta = 1;
+    int stage_level = 0;           // k_pf_multi: 0 = hot tables staged, 1 = + warm, 2 = all (OPFG_HOT/WARM/COLD_TABLES)
     // lane-per-environment kernel: schedule, per-warp scratch in global memory, launch shape
     LaneSchedule lane;
     int pf_kernel = 0;              // OpfgGridDesc.pf_kernel (after the OPFG_PF_KERNEL override)
@@ -1290,6 +1291,7 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
                     if (fit(sizes[lv]) > fit(sizes[level])) level = lv;
             if (const char* sv = getenv("OPFG_STAGE")) level = std::max(0, std::min(2, atoi(sv)));
             d.tab_staged_bytes = sizes[level];
+            G->stage_level = level;
             int E = fit(sizes[level]);
             if (const char* ev = getenv("OPFG_ENVS_PER_CTA")) E = std::min(atoi(ev), E);   // can only lower it
             if (E < 2) E = 1;
@@ -1685,6 +1687,8 @@ int opfg_grid_info(const OpfgGrid* G, OpfgGridInfo* o) {
         o->radial_lanes_per_env = G->tree_T; o->radial_envs_per_cta = G->tree_E;
         o->radial_smem_bytes_per_env = (int)(G->tree_env_doubles * 8);
         o->n_island_critical = G->n_crit;
+        o->cta_envs_per_cta = G->envs_per_cta; o->cta_tables_staged = G->stage_level;
+        o->score_threads_per_env = G->score_threads;
         o->lane_max_row = d.ln_max_row; o->lane_warps_per_cta = G->lane_warps_per_cta; o->lane_tables_staged = G->lane_stage;
         o->lane_scratch_bytes = 8.0 * (double)G->lane_warp_doubles * std::max(1, G->lane_warps_per_cta * G->lane_ctas);
     }
@@ -1941,7 +1945,7 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
             const int n_sm = current_sm_count();
             const int64_t groups = (B->n_env + E - 1) / E;
             const unsigned grid = (unsigned)std::min<int64_t>(groups, n_sm);
-            const int stage = G->d.tab_staged_bytes == G->d.tab_bytes ? 2 : (G->d.tab_staged_bytes == G->d.tab_warm_bytes ? 1 : 0);
+            const int stage = G->stage_level;
             const GridDev view = staged_view(G->d, stage);
             const int env_doubles = (int)(smem / 8);
             void (*fn)(GridDev, OpfgBatch, int, int) = nullptr;
