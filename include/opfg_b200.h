@@ -187,6 +187,14 @@ typedef struct {
     const int32_t* obs_ptr;          /* host [n_obs+1] or NULL: observation j is the SUM of
                                         obs_ref[obs_ptr[j] .. obs_ptr[j+1]) (bus_wise_obs,
                                         opf_env.py:535-536, 806-810)                    */
+    /* three-winding transformers (net.trafo3w): three branch rows each, hv->star, star->mv, star->lv, whose
+       branch_loading_slot entries point at three consecutive result cells and whose rate_f / rate_t are 0 at the
+       star end, so that each cell holds the loading at the outer end of its row.  Kernel 5 then writes
+       res_trafo3w.loading_percent = the largest of the three, NaN if any of them is NaN.
+       n_trafo3w = 0: none (the pointers may be NULL). */
+    int32_t n_trafo3w;
+    const int32_t* trafo3w_row_slot;     /* host [n_trafo3w] first of the 3 S columns of the rows' loadings (hv, mv, lv) */
+    const int32_t* trafo3w_loading_slot; /* host [n_trafo3w] S column of res_trafo3w.loading_percent                     */
 } OpfgScoringDesc;
 
 /* per-environment branch parameters (tap_pos / in_service actions, N-1 contingencies): the listed

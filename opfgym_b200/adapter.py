@@ -6,8 +6,8 @@ solver to fill ``net.res_*`` in place or raise ``LoadflowNotConverged``
 (``opfgym/opf_env.py:53,70,646-662``).  ``power_flow_solver(net)`` does exactly
 that with a batch of ONE environment: kernel 1 scatters the net's injections,
 kernels 2-4 solve, kernel 5 produces the result cells, which are copied back
-into ``res_bus / res_line / res_trafo / res_ext_grid / res_gen / res_load /
-res_sgen / res_storage``.  The compiled grid is cached per net object; the
+into ``res_bus / res_line / res_trafo / res_trafo3w / res_ext_grid / res_gen /
+res_load / res_sgen / res_storage``.  The compiled grid is cached per net object; the
 topology (switches, in_service) is read at first use.
 
 A batch of one cannot be fast (one CTA on a 148-SM part) -- this adapter exists
@@ -30,7 +30,8 @@ _INPUTS = (("load", "p_mw"), ("load", "q_mvar"), ("sgen", "p_mw"), ("sgen", "q_m
            ("storage", "p_mw"), ("storage", "q_mvar"), ("gen", "p_mw"))
 _RESULTS = (("res_bus", "vm_pu"), ("res_bus", "va_degree"), ("res_line", "loading_percent"),
             ("res_trafo", "loading_percent"), ("res_line", "_flows4"), ("res_trafo", "_flows4"),
-            ("res_ext_grid", "p_mw"), ("res_ext_grid", "q_mvar"), ("res_gen", "q_mvar"))
+            ("res_ext_grid", "p_mw"), ("res_ext_grid", "q_mvar"), ("res_gen", "q_mvar"),
+            ("res_trafo3w", "loading_percent"), ("res_trafo3w", "_flows12"))
 
 
 class PowerFlowSolver:
@@ -43,7 +44,7 @@ class PowerFlowSolver:
         self.builder = builder or PpcBuilder(net)
         comp = Compiler(net, self.builder)
         inputs = [(t, c, net[t].index) for t, c in _INPUTS if len(net[t])]
-        results = [(t, c) for t, c in _RESULTS if len(net[t[4:]]) or t == "res_bus"]
+        results = [(t, c) for t, c in _RESULTS if t == "res_bus" or (t[4:] in net and len(net[t[4:]]))]
         self.program = comp.compile(act_keys=[], obs_keys=[], state_keys=inputs, constraints=[],
                                     reward_function=reward_mod.Summation(), extra_results=results)
         from .engine import check_engine_class
@@ -80,6 +81,15 @@ class PowerFlowSolver:
                 f"p_{a}_mw": f4[:, 0], f"q_{a}_mvar": f4[:, 1], f"p_{b}_mw": f4[:, 2],
                 f"q_{b}_mvar": f4[:, 3], "pl_mw": f4[:, 0] + f4[:, 2], "ql_mvar": f4[:, 1] + f4[:, 3],
                 "loading_percent": cells("res_" + table, "loading_percent")}, index=net[table].index)
+        if "trafo3w" in net and len(net.trafo3w):
+            # per winding branch p/q at its from and to end; the outer ends: hv from, mv / lv to
+            f12 = cells("res_trafo3w", "_flows12").reshape(-1, 3, 4)
+            f6 = np.stack([f12[:, 0, 0], f12[:, 0, 1], f12[:, 1, 2], f12[:, 1, 3], f12[:, 2, 2], f12[:, 2, 3]], axis=1)
+            net.res_trafo3w = pd.DataFrame({
+                "p_hv_mw": f6[:, 0], "q_hv_mvar": f6[:, 1], "p_mv_mw": f6[:, 2], "q_mv_mvar": f6[:, 3],
+                "p_lv_mw": f6[:, 4], "q_lv_mvar": f6[:, 5], "pl_mw": f6[:, 0] + f6[:, 2] + f6[:, 4],
+                "ql_mvar": f6[:, 1] + f6[:, 3] + f6[:, 5],
+                "loading_percent": cells("res_trafo3w", "loading_percent")}, index=net.trafo3w.index)
         net.res_ext_grid = pd.DataFrame({"p_mw": cells("res_ext_grid", "p_mw"),
                                          "q_mvar": cells("res_ext_grid", "q_mvar")},
                                         index=net.ext_grid.index)

@@ -72,7 +72,8 @@ class ScoringDesc(C.Structure):
                 ("penalty_factor", C.c_double), ("penalty_bias", C.c_double),
                 ("valid_reward", C.c_double), ("invalid_penalty", C.c_double),
                 ("invalid_objective_share", C.c_double),
-                ("n_obs", C.c_int32), ("obs_ref", _ip), ("obs_ptr", _ip)]
+                ("n_obs", C.c_int32), ("obs_ref", _ip), ("obs_ptr", _ip),
+                ("n_trafo3w", C.c_int32), ("trafo3w_row_slot", _ip), ("trafo3w_loading_slot", _ip)]
 
 
 class DynBranchDesc(C.Structure):

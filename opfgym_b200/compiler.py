@@ -128,12 +128,12 @@ class Compiler:
         v = self.net[table][column].iloc[int(pos)]
         return self.consts.ref(np.nan if v is None else v)
 
-    def _absent_branch_value(self, table, pos) -> float:
+    def _absent_branch_value(self, table, pos, ends=None) -> float:
         """pandapower's result of a branch that is out of service: its rows of ppc['branch'] are never written, so
         flows are 0 and the current 0 / |V| -- 0 between energised buses, NaN if an end bus was dropped
         (results_branch.py `_get_branch_flows` [ext-mem])."""
         net, lk = self.net, self.ppc.bus_lookup
-        ends = ("from_bus", "to_bus") if table == "line" else ("hv_bus", "lv_bus")
+        ends = ends or (("from_bus", "to_bus") if table == "line" else ("hv_bus", "lv_bus"))
         pos_of = {int(b): i for i, b in enumerate(net.bus.index)}
         live = all(lk[pos_of[int(net[table][c].iloc[pos])]] >= 0 for c in ends)
         return 0.0 if live else float("nan")
@@ -204,6 +204,9 @@ class Compiler:
         absent_cells = {}      # result cells of branches that are not in the ppc: 0 between live buses, else NaN
         gen_p_slot = -np.ones(ng, dtype=_I32)
         gen_q_slot = -np.ones(ng, dtype=_I32)
+        n_t3 = len(ppc.trafo3w_branch)
+        t3_loading_slot = -np.ones(n_t3, dtype=_I32)
+        t3_row_slot = -np.ones(n_t3, dtype=_I32)
         for table, column in sorted(wanted):
             base = table[len(RES_PREFIX):]
             n_rows = len(net[base])
@@ -242,8 +245,33 @@ class Compiler:
                     else:
                         for k in range(4):
                             absent_cells[start + 4 * pos + k] = self._absent_branch_value(base, pos)
-            elif table == "res_trafo3w":
-                lay.add(table, column, n_rows)   # no trafo3w model: column stays NaN
+            elif table == "res_trafo3w" and column == "loading_percent":
+                # kernel 5: the branch loop writes the outer-end loading of each of the three star branches into
+                # three hidden cells (the star ends have factor 0), then one lane per element takes their max.  A
+                # winding whose branch is absent is 0 next to a live bus and NaN next to a dropped one
+                # (PANDAPOWER_ASSUMPTIONS 16): a constant cell
+                start = lay.add(table, column, n_rows)
+                rows3 = lay.add(table, "_rows3", 3 * n_rows)
+                for pos in range(n_rows):
+                    t3_loading_slot[pos] = start + pos
+                    t3_row_slot[pos] = rows3 + 3 * pos
+                    for w, (side, br) in enumerate(zip(("hv", "mv", "lv"), ppc.trafo3w_branch[pos])):
+                        if br >= 0:
+                            loading_slot[br] = rows3 + 3 * pos + w
+                        else:
+                            absent_cells[rows3 + 3 * pos + w] = self._absent_branch_value("trafo3w", pos, (f"{side}_bus",))
+            elif table == "res_trafo3w" and column == "_flows12":
+                # 4 cells per winding branch, as for res_trafo _flows4 (adapter only): the outer end is the hv
+                # branch's from end and the mv / lv branches' to end
+                start = lay.add(table, column, 12 * n_rows)
+                for pos in range(n_rows):
+                    for w, (side, br) in enumerate(zip(("hv", "mv", "lv"), ppc.trafo3w_branch[pos])):
+                        if br >= 0:
+                            flow_slot[br] = start + 12 * pos + 4 * w
+                        else:
+                            for k in range(4):
+                                absent_cells[start + 12 * pos + 4 * w + k] = \
+                                    self._absent_branch_value("trafo3w", pos, (f"{side}_bus",))
             elif table in ("res_load", "res_sgen", "res_storage", "res_gen") and column in ("p_mw", "q_mvar"):
                 pass   # = set-point * scaling, referenced with a multiplier (no cell needed)
             else:
@@ -473,6 +501,24 @@ class Compiler:
                              float(tr.tap_step_percent.iloc[pos]),
                              float(self.builder.trafo_ratio_neutral[k]), svc,
                              sw_ends.get(("trafo", pos, 0), one), sw_ends.get(("trafo", pos, 1), one), flags))
+        if lay.has("trafo3w", "in_service"):
+            raise NotImplementedError("trafo3w.in_service as a per-environment cell is not modelled")
+        if lay.has("trafo3w", "tap_pos"):
+            # the tapped winding's equivalent branch is a 2-winding transformer: kernel 1's trafo tap math
+            # applies, on its HV or LV end (PANDAPOWER_ASSUMPTIONS 14)
+            t3 = net.trafo3w
+            if not hasattr(self.builder, "trafo3w_tap_w"):
+                raise NotImplementedError("per-environment trafo3w.tap_pos needs the in-repo net conversion (PpcBuilder)")
+            for pos, rows in enumerate(ppc.trafo3w_branch):
+                w = int(self.builder.trafo3w_tap_w[pos])
+                if w < 0 or rows[w] < 0:
+                    continue           # no tap changer (pandapower ignores tap_pos then), or the branch is absent
+                br = int(rows[w])
+                k = br - self.builder.trafo3w_first          # position in the builder's trafo3w rows
+                flags = capi_flags.DYN_TRAFO | (capi_flags.DYN_TAP_LV if self.builder.trafo3w_tap_at_lv[pos] else 0)
+                dyn_rows.append((br, self.value_ref("trafo3w", "tap_pos", pos), float(t3.tap_neutral.iloc[pos]),
+                                 float(t3.tap_step_percent.iloc[pos]), float(self.builder.trafo3w_ratio_neutral[k]),
+                                 one, one, one, flags))
         if dyn_rows:
             cols = list(zip(*dyn_rows))
             dyn = dict(branch=np.asarray(cols[0], _I32), tap_pos=np.asarray(cols[1], _I32),
@@ -500,7 +546,9 @@ class Compiler:
             n_pwl=len(pw), n_pwl_seg=n_seg, pwl_v=np.asarray(pwl_v, _I32),
             pwl_v_mul=np.asarray(pwl_vm, float), pwl_seg=np.asarray(pwl_seg, _I32),
             reward=rp, n_obs=len(obs_ptr) - 1, obs_ref=np.asarray(obs_ref, _I32),
-            obs_ptr=np.asarray(obs_ptr, _I32) if len(obs_ref) != len(obs_ptr) - 1 else None)
+            obs_ptr=np.asarray(obs_ptr, _I32) if len(obs_ref) != len(obs_ptr) - 1 else None,
+            n_trafo3w=n_t3 if (t3_loading_slot >= 0).any() else 0,
+            trafo3w_row_slot=t3_row_slot, trafo3w_loading_slot=t3_loading_slot)
 
         return EnvProgram(ppc=ppc, layout=lay, consts=np.asarray(self.consts.values, float),
                           initial_state=init, assembly=assembly, scoring=scoring,
@@ -585,7 +633,10 @@ def fill_descs(capi, program: EnvProgram, tol_pu, max_iter, init_dc, enforce_q_l
         objective_bias=r["objective_bias"], penalty_factor=r["penalty_factor"],
         penalty_bias=r["penalty_bias"], valid_reward=r["valid_reward"],
         invalid_penalty=r["invalid_penalty"], invalid_objective_share=r["invalid_objective_share"],
-        n_obs=s["n_obs"], obs_ref=iptr(s["obs_ref"]), obs_ptr=iptr(s["obs_ptr"]))
+        n_obs=s["n_obs"], obs_ref=iptr(s["obs_ref"]), obs_ptr=iptr(s["obs_ptr"]),
+        n_trafo3w=s["n_trafo3w"])
+    if s["n_trafo3w"]:
+        sd.trafo3w_row_slot, sd.trafo3w_loading_slot = iptr(s["trafo3w_row_slot"]), iptr(s["trafo3w_loading_slot"])
     dd = None
     if program.dyn_branches is not None:
         d = program.dyn_branches

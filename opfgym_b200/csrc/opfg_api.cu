@@ -1588,7 +1588,8 @@ int opfg_set_scoring(OpfgGrid* G, const OpfgScoringDesc* sc) {
         {
             const size_t cap = 8192 + 16 * (size_t)sc->n_pp_bus + 96 * (size_t)nbr + 32 * (size_t)ng + 48 * (size_t)n_el +
                                64 * (size_t)sc->n_constraints + 64 * (size_t)sc->n_poly + 32 * (size_t)sc->n_pwl * (sc->n_pwl_seg + 1) +
-                               8 * (size_t)sc->n_obs + 8 * G->consts_host.size() + 16 * (size_t)d.nb;
+                               8 * (size_t)sc->n_obs + 8 * G->consts_host.size() + 16 * (size_t)d.nb +
+                               (sc->n_trafo3w > 0 ? 32 + 8 * (size_t)sc->n_trafo3w : 0);
             G->tab2_base = (char*)dev_alloc(cap);
             if (!G->tab2_base) throw std::runtime_error("device allocation failed");
             G->allocs.push_back(G->tab2_base);
@@ -1600,6 +1601,20 @@ int opfg_set_scoring(OpfgGrid* G, const OpfgScoringDesc* sc) {
         d.br_loading_slot = G->tab2(sc->branch_loading_slot, nbr);
         d.br_flow_slot = G->tab2(sc->branch_flow_slot, nbr);
         d.rate_f = G->tab2(sc->rate_f, nbr); d.rate_t = G->tab2(sc->rate_t, nbr);
+        d.n_t3 = 0; d.t3_row_slot = d.t3_loading_slot = nullptr;
+        if (sc->n_trafo3w < 0) throw std::runtime_error("n_trafo3w < 0");
+        if (sc->n_trafo3w > 0) {
+            const int n3 = sc->n_trafo3w;
+            if (!sc->trafo3w_row_slot || !sc->trafo3w_loading_slot) throw std::runtime_error("trafo3w tables missing");
+            for (int k = 0; k < n3; ++k) {
+                const int rs = sc->trafo3w_row_slot[k], ls = sc->trafo3w_loading_slot[k];
+                if (rs < sc->n_inputs || rs + 3 > d.n_state || ls < sc->n_inputs || ls >= d.n_state)
+                    throw std::runtime_error("trafo3w result slot out of range");
+            }
+            d.n_t3 = n3;
+            d.t3_row_slot = G->tab2(sc->trafo3w_row_slot, n3);
+            d.t3_loading_slot = G->tab2(sc->trafo3w_loading_slot, n3);
+        }
         d.gen_bus = G->tab2(G->gen_bus_host);
         d.gen_q_share = G->tab2(G->gen_q_share_host);
         d.gen_p_slot = G->tab2(sc->gen_p_slot, ng); d.gen_q_slot = G->tab2(sc->gen_q_slot, ng);
@@ -1655,6 +1670,7 @@ int opfg_set_scoring(OpfgGrid* G, const OpfgScoringDesc* sc) {
         if (d.res_va_slot >= 0) cells += d.n_pp_bus;
         for (int l = 0; l < nbr; ++l) cells += (sc->branch_loading_slot[l] >= 0) + 4 * (sc->branch_flow_slot[l] >= 0);
         for (int gI = 0; gI < ng; ++gI) cells += (sc->gen_p_slot[gI] >= 0) + (sc->gen_q_slot[gI] >= 0);
+        cells += sc->n_trafo3w;       // res_trafo3w.loading_percent (its rows' cells are counted with the branches)
         G->n_result_cells = cells;
         G->flops_score = 60.0 * nbr + 30.0 * d.nb + 10.0 * n_el + 14.0 * d.n_poly + 20.0 * d.n_pwl * d.n_pwl_seg + 40.0;
         {   // one warp per environment on small grids: reductions are pure shuffles, no barriers

@@ -112,6 +112,8 @@ struct GridDev {
     const int* pp_lookup;
     const int *br_loading_slot, *br_flow_slot;
     const double *rate_f, *rate_t;
+    int n_t3;                          // three-winding transformers (OpfgScoringDesc.trafo3w_*)
+    const int *t3_row_slot, *t3_loading_slot;
     const int *gen_bus, *gen_p_slot, *gen_q_slot;
     const double* gen_q_share;
     int n_con;
@@ -1624,6 +1626,20 @@ OPFG_HD void env_score(const GridDev& g, const C& cx, double* smem, const OpfgBa
 #ifdef OPFG_DEVICE_BUILD
     __threadfence_block();
 #endif
+    if (g.n_t3 > 0) {
+        // three-winding transformers (results_branch.py _get_trafo3w_results [ext-mem]): the branch loop above
+        // left the loading at the outer end of each of the three star branches in three consecutive cells (the
+        // star ends have factor 0); one element per lane takes the largest, NaN if any is NaN (numpy's max)
+        for (int k = cx.tid; k < g.n_t3; k += T) {
+            const double* c = S + g.t3_row_slot[k];
+            const double a = c[0], b = c[1], d = c[2];
+            S[g.t3_loading_slot[k]] = (a != a || b != b || d != d) ? NAN : fmax(a, fmax(b, d));
+        }
+        cx.sync();
+#ifdef OPFG_DEVICE_BUILD
+        __threadfence_block();
+#endif
+    }
     // constraints (opfgym/constraints.py:70-128)
     double pen_sum = 0;
     bool all_valid = true;

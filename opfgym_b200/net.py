@@ -29,7 +29,12 @@ _TABLES = {
               "shift_degree", "tap_side", "tap_neutral", "tap_min", "tap_max",
               "tap_step_percent", "tap_step_degree", "tap_pos", "parallel",
               "df", "in_service"],
-    "trafo3w": ["name", "hv_bus", "mv_bus", "lv_bus", "in_service"],
+    "trafo3w": ["name", "hv_bus", "mv_bus", "lv_bus", "sn_hv_mva", "sn_mv_mva", "sn_lv_mva",
+                "vn_hv_kv", "vn_mv_kv", "vn_lv_kv", "vk_hv_percent", "vk_mv_percent",
+                "vk_lv_percent", "vkr_hv_percent", "vkr_mv_percent", "vkr_lv_percent",
+                "pfe_kw", "i0_percent", "shift_mv_degree", "shift_lv_degree", "tap_side",
+                "tap_neutral", "tap_min", "tap_max", "tap_step_percent", "tap_step_degree",
+                "tap_pos", "tap_at_star_point", "in_service"],
     "load": ["name", "bus", "p_mw", "q_mvar", "const_z_percent",
              "const_i_percent", "scaling", "in_service"],
     "sgen": ["name", "bus", "p_mw", "q_mvar", "scaling", "in_service"],
@@ -55,7 +60,8 @@ _RES_TABLES = {
     "res_trafo": ["p_hv_mw", "q_hv_mvar", "p_lv_mw", "q_lv_mvar", "pl_mw",
                   "ql_mvar", "i_hv_ka", "i_lv_ka", "vm_hv_pu", "vm_lv_pu",
                   "loading_percent"],
-    "res_trafo3w": ["loading_percent"],
+    "res_trafo3w": ["p_hv_mw", "q_hv_mvar", "p_mv_mw", "q_mv_mvar", "p_lv_mw", "q_lv_mvar",
+                    "pl_mw", "ql_mvar", "loading_percent"],
     "res_ext_grid": ["p_mw", "q_mvar"],
     "res_load": ["p_mw", "q_mvar"],
     "res_sgen": ["p_mw", "q_mvar"],
@@ -84,7 +90,7 @@ class Net:
             for c in df.columns:
                 if c in ("name", "type", "tap_side", "et", "power_type", "points"):
                     df[c] = df[c].astype(object)
-                elif c in ("in_service", "closed", "slack"):
+                elif c in ("in_service", "closed", "slack", "tap_at_star_point"):
                     df[c] = df[c].astype(bool)
                 elif c in ("bus", "from_bus", "to_bus", "hv_bus", "lv_bus",
                            "mv_bus", "element"):
@@ -145,7 +151,7 @@ _DEFAULTS = {
     "name": None, "in_service": True, "scaling": 1.0, "parallel": 1.0,
     "df": 1.0, "g_us_per_km": 0.0, "const_z_percent": 0.0,
     "const_i_percent": 0.0, "q_mvar": 0.0, "type": "b", "va_degree": 0.0,
-    "slack": False, "tap_step_degree": 0.0, "step": 1.0, "closed": True,
+    "slack": False, "tap_step_degree": 0.0, "tap_at_star_point": False, "step": 1.0, "closed": True,
     "min_q_mvar": np.nan, "max_q_mvar": np.nan,
     "cp0_eur": 0.0, "cp1_eur_per_mw": 0.0, "cp2_eur_per_mw2": 0.0,
     "cq0_eur": 0.0, "cq1_eur_per_mvar": 0.0, "cq2_eur_per_mvar2": 0.0,
@@ -204,6 +210,38 @@ def create_transformer_from_parameters(net, hv_bus, lv_bus, sn_mva, vn_hv_kv,
                 tap_step_percent=[tap_step_percent], tap_pos=[tap_pos])
     data.update({k: [v] for k, v in cols.items()})
     return int(_bulk(net, "trafo", data)[0])
+
+
+def create_transformer3w_from_parameters(net, hv_bus, mv_bus, lv_bus, vn_hv_kv, vn_mv_kv, vn_lv_kv,
+                                         sn_hv_mva, sn_mv_mva, sn_lv_mva, vk_hv_percent, vk_mv_percent,
+                                         vk_lv_percent, vkr_hv_percent, vkr_mv_percent, vkr_lv_percent,
+                                         pfe_kw, i0_percent, shift_mv_degree=0.0, shift_lv_degree=0.0,
+                                         tap_side=None, tap_step_percent=np.nan, tap_step_degree=np.nan,
+                                         tap_pos=np.nan, tap_neutral=np.nan, tap_max=np.nan, tap_min=np.nan,
+                                         name=None, in_service=True, index=None, max_loading_percent=np.nan,
+                                         tap_at_star_point=False, **cols) -> int:
+    """Same call shape as ``pp.create_transformer3w_from_parameters``.  The short-circuit voltages are
+    pairwise: ``vk_hv_percent`` hv-mv, ``vk_mv_percent`` mv-lv, ``vk_lv_percent`` hv-lv."""
+    if np.isnan(tap_pos) and not np.isnan(tap_neutral):
+        tap_pos = tap_neutral
+    data = dict(hv_bus=[int(hv_bus)], mv_bus=[int(mv_bus)], lv_bus=[int(lv_bus)],
+                sn_hv_mva=[sn_hv_mva], sn_mv_mva=[sn_mv_mva], sn_lv_mva=[sn_lv_mva],
+                vn_hv_kv=[vn_hv_kv], vn_mv_kv=[vn_mv_kv], vn_lv_kv=[vn_lv_kv],
+                vk_hv_percent=[vk_hv_percent], vk_mv_percent=[vk_mv_percent], vk_lv_percent=[vk_lv_percent],
+                vkr_hv_percent=[vkr_hv_percent], vkr_mv_percent=[vkr_mv_percent],
+                vkr_lv_percent=[vkr_lv_percent], pfe_kw=[pfe_kw], i0_percent=[i0_percent],
+                shift_mv_degree=[shift_mv_degree], shift_lv_degree=[shift_lv_degree], tap_side=[tap_side],
+                tap_neutral=[tap_neutral], tap_min=[tap_min], tap_max=[tap_max],
+                tap_step_percent=[tap_step_percent], tap_step_degree=[tap_step_degree], tap_pos=[tap_pos],
+                tap_at_star_point=[bool(tap_at_star_point)], in_service=[bool(in_service)], name=[name])
+    if not np.isnan(max_loading_percent):
+        data["max_loading_percent"] = [float(max_loading_percent)]
+    data.update({k: [v] for k, v in cols.items()})
+    out = int(_bulk(net, "trafo3w", data)[0])
+    if index is not None:
+        net.trafo3w = net.trafo3w.rename(index={out: int(index)})
+        out = int(index)
+    return out
 
 
 def _create_pq(net, table, buses, p_mw, q_mvar, **cols) -> np.ndarray:

@@ -18,6 +18,10 @@ pandapower's private attributes is marked [ext-mem] (from memory of pandapower 2
 * gen rows: ext_grids in table order first, then gens (``build_gen.py``); cross-checked through the bus.
 * the shunt branch admittance: complex ``BR_B`` (``y = 1j * BR_B``) in pandapower < 2.14, a separate real
   ``BR_G`` column afterwards.
+* ``net._pd2ppc_lookups["branch"]["trafo3w"]``: 3 rows per element, in blocks -- every element's hv->star row,
+  then every mv row (star->mv), then every lv row (star->lv) (``build_branch._trafo_df_from_trafo3w``).  Loading
+  of element k is the largest of the three outer-end currents (hv: the row's from bus, mv / lv: its to bus), each
+  scaled by ``vn_<side>_kv / sn_<side>_mva`` (``results_branch._get_trafo3w_results``).
 """
 from __future__ import annotations
 
@@ -118,13 +122,29 @@ class PandapowerPpcBuilder:
                 cap = float(tr.sn_mva) * float(tr.parallel) * float(tr.df)
                 rate_f[r] = float(tr.vn_hv_kv) / (base_kv[int(branch[r, P.F_BUS])] * cap)
                 rate_t[r] = float(tr.vn_lv_kv) / (base_kv[int(branch[r, P.T_BUS])] * cap)
-        # Branches of other element tables (trafo3w: three rows each behind an auxiliary bus; impedance) are solved
-        # like any other row of pandapower's ppc; they have no result rows here (no res_trafo3w / res_impedance cells,
-        # loading factors 0).  An xward also injects power at its bus, which kernel 1 would not scatter: rejected.
+        # trafo3w: three rows per element behind its star-point bus, loading factors at the outer ends only
+        n3 = len(net.trafo3w) if "trafo3w" in net else 0
+        self.trafo3w_branch = -np.ones((n3, 3), dtype=np.int64)
+        if n3 and "trafo3w" in ranges:
+            a, b = ranges["trafo3w"]
+            if b - a != 3 * n3:
+                raise RuntimeError("net._ppc['branch'] does not hold 3 rows per trafo3w [ext-mem]")
+            self.trafo3w_branch[:] = row_of[a:b].reshape(3, n3).T
+            for pos, rows in enumerate(self.trafo3w_branch):
+                t3 = net.trafo3w.iloc[pos]
+                for w, (side, end) in enumerate((("hv", P.F_BUS), ("mv", P.T_BUS), ("lv", P.T_BUS))):
+                    r = rows[w]
+                    if r < 0:
+                        continue
+                    rate = float(t3[f"vn_{side}_kv"]) / (base_kv[int(branch[r, end])] * float(t3[f"sn_{side}_mva"]))
+                    (rate_f if end == P.F_BUS else rate_t)[r] = rate
+        # Branches of other element tables (impedance) are solved like any other row of pandapower's ppc; they have
+        # no result rows here (no res_impedance cells, loading factors 0).  An xward also injects power at its bus,
+        # which kernel 1 would not scatter: rejected.
         self.other_branch_rows = {}
-        covered = (self.line_branch >= 0).sum() + (self.trafo_branch >= 0).sum()
+        covered = (self.line_branch >= 0).sum() + (self.trafo_branch >= 0).sum() + (self.trafo3w_branch >= 0).sum()
         for table in ranges:
-            if table in ("line", "trafo"):
+            if table in ("line", "trafo", "trafo3w"):
                 continue
             a, b = ranges[table]
             rows = row_of[a:b][row_of[a:b] >= 0]
@@ -141,7 +161,8 @@ class PandapowerPpcBuilder:
                           bus_lookup=self.bus_lookup.copy(), line_branch=self.line_branch.copy(),
                           trafo_branch=self.trafo_branch.copy(), ext_grid_gen=self.ext_grid_gen,
                           gen_gen=self.gen_gen, rate_f=rate_f, rate_t=rate_t,
-                          init_vm_pu=float(vm.mean()) if len(vm) else 1.0)
+                          init_vm_pu=float(vm.mean()) if len(vm) else 1.0,
+                          trafo3w_branch=self.trafo3w_branch.copy())
 
     def element_bus(self, net, table):
         pos = np.array([self._pos_of[int(b)] for b in net[table].bus.to_numpy()], dtype=np.int64)

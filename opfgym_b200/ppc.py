@@ -38,6 +38,25 @@ oracle/pf.py (none could be checked here: pandapower is not installed):
     per-unit mismatch (identical for sn_mva=1, the SimBench value).
  7. enforce_q_lims skips generators whose QMIN and QMAX are both 0.
  8. trafo_loading='current'.
+ 9. trafo3w (build_branch._trafo_df_from_trafo3w): one auxiliary star-point bus and three 2-winding
+    equivalent branches hv->star, star->mv, star->lv, stacked behind the trafos in three blocks (all hv
+    rows, all mv rows, all lv rows) and before the impedances.
+10. trafo3w vk_hv/mv/lv_percent and vkr_* are the pairwise hv-mv, mv-lv and hv-lv values; each pair is
+    referred to sn_hv_mva through min(sn) of its two windings (z_br_to_bus_vector), then converted
+    delta->star separately for the real part and the reactance: z_i = 0.5*sn_i/sn_hv*(z_ij+z_ik-z_jk)
+    (wye_delta_vector); vk_i = sign(x_i)*sqrt(x_i^2+r_i^2), so a star impedance may be negative.
+11. equivalent branch i has sn = sn_<i>_mva, vn_hv_kv = vn_hv_kv, vn_lv_kv = vn_<i>_kv, parallel = df = 1,
+    and is then converted like a trafo (item 4).
+12. trafo3w_losses='hv': pfe_kw and i0_percent sit on the hv branch only.
+13. shift_mv_degree on the mv branch, shift_lv_degree on the lv branch, none on the hv branch.
+14. the trafo3w tap changer sits on the branch of the winding named by tap_side, at its outer end
+    (hv branch: hv side; mv / lv branch: lv side); with tap_at_star_point at the star end of that
+    branch instead.  tap_step_degree != 0 (phase shifter) is not modelled.
+15. the star bus has the hv bus's nominal voltage as base kV.
+16. res_trafo3w.loading_percent (trafo_loading='current', _get_trafo3w_results) = max(ld_hv, ld_mv, ld_lv),
+    ld_i = current at the outer bus of branch i * vn_<i>_kv / sn_<i>_mva * sqrt3 * 100 (star ends are not
+    counted), numpy's NaN-propagating max; an absent branch contributes 0 next to a live bus, NaN next to a
+    dropped one.
 """
 
 # PYPOWER column indices
@@ -65,6 +84,9 @@ class Ppc:
     init_vm_pu: float = 1.0
     meta: dict = field(default_factory=dict)
     impedance_branch: np.ndarray = field(default_factory=lambda: np.zeros(0, np.int64))  # net.impedance position -> branch row
+    # net.trafo3w position -> branch rows of its hv->star, star->mv, star->lv equivalents (-1: out).  Their loading
+    # factors sit at the outer end (rate_f of the hv row, rate_t of the mv / lv rows); the star ends have 0.
+    trafo3w_branch: np.ndarray = field(default_factory=lambda: np.zeros((0, 3), np.int64))
 
     @property
     def nb(self):
@@ -91,8 +113,72 @@ class _DSU:
                 self.p[ra] = rb
 
 
-UNSUPPORTED_TABLES = ("trafo3w", "xward", "dcline", "motor", "asymmetric_load",
+UNSUPPORTED_TABLES = ("xward", "dcline", "motor", "asymmetric_load",
                       "asymmetric_sgen", "svc", "tcsc", "ssc", "vsc")
+
+
+TRAFO3W_COLUMNS = ("hv_bus", "mv_bus", "lv_bus", "sn_hv_mva", "sn_mv_mva", "sn_lv_mva", "vn_hv_kv", "vn_mv_kv",
+                   "vn_lv_kv", "vk_hv_percent", "vk_mv_percent", "vk_lv_percent", "vkr_hv_percent", "vkr_mv_percent",
+                   "vkr_lv_percent", "pfe_kw", "i0_percent", "shift_mv_degree", "shift_lv_degree", "tap_side",
+                   "tap_neutral", "tap_step_percent", "tap_pos", "in_service")
+
+
+def trafo_branch_values(vn_hv, vn_lv, vn_hv_bus, vn_lv_bus, sn_t, vk, vkr, pfe_kw, i0, steps, on_hv, on_lv, par,
+                        sn, trafo_model):
+    """2-winding transformer -> pi branch (pandapower build_branch ``_calc_branch_values_from_trafo_df``
+    [ext-mem]), on arrays.  Returns r, x, g, b, ratio and the ratio at the neutral tap."""
+    vnh = np.where(on_hv, vn_hv * (1.0 + steps), vn_hv)
+    vnl = np.where(on_lv, vn_lv * (1.0 + steps), vn_lv)
+    ratio = (vnh / vnl) / (vn_hv_bus / vn_lv_bus)
+    ratio_neutral = (vn_hv / vn_lv) / (vn_hv_bus / vn_lv_bus)
+    # short-circuit impedance, referred to the LV bus voltage
+    tap_lv = (vnl / vn_lv_bus) ** 2 * sn
+    z_sc = vk / 100.0 / sn_t * tap_lv
+    r_sc = vkr / 100.0 / sn_t * tap_lv
+    x_sc = np.sign(z_sc) * np.sqrt(z_sc ** 2 - r_sc ** 2)
+    r = r_sc / par
+    x = x_sc / par
+    # magnetising branch
+    base_r = vn_lv_bus ** 2 / sn
+    vnl_sq = vn_lv ** 2
+    pfe = pfe_kw * 1e-3
+    g_m = pfe / vnl_sq * base_r
+    b_sq = (i0 / 100.0 * sn_t) ** 2 - pfe ** 2
+    b_sq[b_sq < 0] = 0.0
+    b_m = np.sqrt(b_sq) * base_r / vnl_sq * np.sign(i0)
+    y_sh = (g_m - 1j * b_m) / (vnl / vn_lv) ** 2 * par
+    if trafo_model == "t":
+        nz = y_sh != 0
+        za = (r[nz] + 1j * x[nz]) / 2.0
+        zc = 1.0 / y_sh[nz]
+        zsum = za * za + 2.0 * za * zc
+        zab = zsum / zc
+        zbc = zsum / za
+        r = r.copy()
+        x = x.copy()
+        r[nz], x[nz] = zab.real, zab.imag
+        y_sh = y_sh.copy()
+        y_sh[nz] = 2.0 / zbc
+    return r, x, y_sh.real, y_sh.imag, ratio, ratio_neutral
+
+
+def trafo3w_star_parameters(t3):
+    """Star-equivalent (vk, vkr) [%] of every trafo3w, each row [hv, mv, lv] on its own sn_<side>_mva
+    (pandapower ``_calculate_sc_voltages_of_equivalent_transformers`` [ext-mem])."""
+    sn = np.stack([t3.sn_hv_mva.to_numpy(float), t3.sn_mv_mva.to_numpy(float), t3.sn_lv_mva.to_numpy(float)])
+
+    def to_hv_base(z):          # pairs hv-mv, mv-lv, hv-lv, each referred to sn_hv through min(sn) of the pair
+        return sn[0] * np.array([z[0] / np.minimum(sn[0], sn[1]), z[1] / np.minimum(sn[1], sn[2]),
+                                 z[2] / np.minimum(sn[0], sn[2])])
+
+    def delta_to_star(z):
+        return 0.5 * sn / sn[0] * np.array([z[0] + z[2] - z[1], z[1] + z[0] - z[2], z[2] + z[1] - z[0]])
+
+    vk = to_hv_base(np.stack([t3[f"vk_{s}_percent"].to_numpy(float) for s in ("hv", "mv", "lv")]))
+    vkr = to_hv_base(np.stack([t3[f"vkr_{s}_percent"].to_numpy(float) for s in ("hv", "mv", "lv")]))
+    vki = np.sqrt(vk ** 2 - vkr ** 2)
+    vkr_s, vki_s = delta_to_star(vkr), delta_to_star(vki)
+    return np.sign(vki_s) * np.sqrt(vki_s ** 2 + vkr_s ** 2), vkr_s, sn
 
 
 class PpcBuilder:
@@ -119,7 +205,18 @@ class PpcBuilder:
             if df is not None and len(df):
                 raise NotImplementedError(
                     f"net.{table} has {len(df)} rows: {table} elements are not modelled by PpcBuilder "
-                    "(supported: bus, line, trafo, impedance, switch, load, sgen, storage, ward, gen, ext_grid, shunt)")
+                    "(supported: bus, line, trafo, trafo3w, impedance, switch, load, sgen, storage, ward, gen, ext_grid, shunt)")
+        t3 = getattr(net, "trafo3w", None) if not isinstance(net, dict) else net.get("trafo3w")
+        if t3 is not None and len(t3):
+            missing = [c for c in TRAFO3W_COLUMNS if c not in t3.columns]
+            if missing:
+                raise NotImplementedError(f"net.trafo3w lacks the parameter columns {missing} of the star-point model")
+            step_deg = np.nan_to_num(t3.tap_step_degree.to_numpy(float))
+            if (step_deg != 0).any():
+                raise NotImplementedError("net.trafo3w with tap_step_degree != 0: phase-shifting tap changers of "
+                                          "three-winding transformers are not modelled")
+            if len(net.switch) and (net.switch.et == "t3").any():
+                raise NotImplementedError("switches at net.trafo3w (et='t3') are not modelled")
         self._analyse(net)
 
     # ------------------------------------------------------------------ topology
@@ -193,7 +290,21 @@ class PpcBuilder:
                 node_t[i] = k
                 aux_vn.append(vn[lt[i]])
             k += 1
-        n_nodes = n_pp + n_aux
+        # three-winding transformers: one star-point node per element, auxiliary like the buses above (a star
+        # that nothing in service reaches is dropped by the connectivity walk)
+        t3 = getattr(net, "trafo3w", None)
+        n3 = len(t3) if t3 is not None else 0
+        if n3:
+            t3_end = np.array([[pos_of[int(b)] for b in t3[c].to_numpy()] for c in ("hv_bus", "mv_bus", "lv_bus")],
+                              dtype=np.int64).T                             # [n3, 3]
+            t3_row_in = t3.in_service.to_numpy(bool)[:, None] & bus_in[t3_end]
+            t3_star = n_pp + n_aux + np.arange(n3)
+            aux_vn.extend(vn[t3_end[:, 0]])
+        else:
+            t3_end = np.zeros((0, 3), np.int64)
+            t3_row_in = np.zeros((0, 3), bool)
+            t3_star = np.zeros(0, np.int64)
+        n_nodes = n_pp + n_aux + n3
 
         # impedance elements (pandapower build_branch._calc_impedance_parameter): plain series branches
         imp = getattr(net, "impedance", None)
@@ -217,6 +328,10 @@ class PpcBuilder:
             adj[node_t[i]].append(node_f[i])
         for i in np.nonzero(t_in)[0]:
             a, b = root[th[i]], root[tl[i]]
+            adj[a].append(b)
+            adj[b].append(a)
+        for k, w in zip(*np.nonzero(t3_row_in)):
+            a, b = t3_star[k], root[t3_end[k, w]]
             adj[a].append(b)
             adj[b].append(a)
         eg_in = net.ext_grid.in_service.to_numpy(bool) if len(net.ext_grid) else np.zeros(0, bool)
@@ -260,13 +375,27 @@ class PpcBuilder:
         self.line_branch[self.line_pos] = np.arange(len(self.line_pos))
         self.trafo_branch = -np.ones(nt, dtype=np.int64)
         self.trafo_branch[self.trafo_pos] = len(self.line_pos) + np.arange(len(self.trafo_pos))
+        # trafo3w rows in pandapower's stacking: every hv row, then every mv row, then every lv row
+        if n3:
+            t3_row_in &= (node_id[t3_star][:, None] >= 0) & (node_id[root[t3_end]] >= 0)
+        self.trafo3w_rows = [(int(k), w) for w in range(3) for k in np.nonzero(t3_row_in[:, w])[0]]
+        star = [int(node_id[t3_star[k]]) for k, _ in self.trafo3w_rows]
+        outer = [int(node_id[root[t3_end[k, w]]]) for k, w in self.trafo3w_rows]
+        self.trafo3w_f = np.array([o if w == 0 else st for (_, w), st, o in zip(self.trafo3w_rows, star, outer)],
+                                  dtype=np.int64)
+        self.trafo3w_t = np.array([st if w == 0 else o for (_, w), st, o in zip(self.trafo3w_rows, star, outer)],
+                                  dtype=np.int64)
+        first3 = self.trafo3w_first = len(self.line_pos) + len(self.trafo_pos)
+        self.trafo3w_branch = -np.ones((n3, 3), dtype=np.int64)
+        for r, (k, w) in enumerate(self.trafo3w_rows):
+            self.trafo3w_branch[k, w] = first3 + r
         if ni:
             i_in &= (node_id[root[imf]] >= 0) & (node_id[root[imt]] >= 0)
         self.imp_pos = np.nonzero(i_in)[0]
         self.imp_f = node_id[root[imf[self.imp_pos]]] if ni else np.zeros(0, np.int64)
         self.imp_t = node_id[root[imt[self.imp_pos]]] if ni else np.zeros(0, np.int64)
         self.impedance_branch = -np.ones(ni, dtype=np.int64)
-        self.impedance_branch[self.imp_pos] = len(self.line_pos) + len(self.trafo_pos) + np.arange(len(self.imp_pos))
+        self.impedance_branch[self.imp_pos] = first3 + len(self.trafo3w_rows) + np.arange(len(self.imp_pos))
         self.n_pp_bus = n_pp
 
     def element_bus(self, net, table) -> np.ndarray:
@@ -278,12 +407,13 @@ class PpcBuilder:
     def branch_table(self, net) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
         sn = net.sn_mva
         nl, nt, ni = len(self.line_pos), len(self.trafo_pos), len(self.imp_pos)
-        br = np.zeros((nl + nt + ni, BRANCH_COLS))
+        n3r = len(self.trafo3w_rows)
+        br = np.zeros((nl + nt + n3r + ni, BRANCH_COLS))
         br[:, TAP] = 1.0
         br[:, BR_STATUS] = 1.0
         br[:, ANGMIN], br[:, ANGMAX] = -360.0, 360.0
-        rate_f = np.zeros(nl + nt + ni)
-        rate_t = np.zeros(nl + nt + ni)
+        rate_f = np.zeros(nl + nt + n3r + ni)
+        rate_t = np.zeros(nl + nt + n3r + ni)
         if nl:
             ln = net.line.iloc[self.line_pos]
             vn_f = self.base_kv[self.line_f]
@@ -305,8 +435,6 @@ class PpcBuilder:
             tr = net.trafo.iloc[self.trafo_pos]
             vn_hv_bus = self.base_kv[self.trafo_h]
             vn_lv_bus = self.base_kv[self.trafo_l]
-            vnh = tr.vn_hv_kv.to_numpy(float).copy()
-            vnl = tr.vn_lv_kv.to_numpy(float).copy()
             # tap changer (ratio only; tap_step_degree == 0)
             tap_pos = tr.tap_pos.to_numpy(float)
             tap_neutral = tr.tap_neutral.to_numpy(float)
@@ -315,50 +443,21 @@ class PpcBuilder:
             side = tr.tap_side.to_numpy(object)
             on_hv = np.array([s == "hv" for s in side])
             on_lv = np.array([s == "lv" for s in side])
-            vnh = np.where(on_hv, vnh * (1.0 + steps), vnh)
-            vnl = np.where(on_lv, vnl * (1.0 + steps), vnl)
-            ratio = (vnh / vnl) / (vn_hv_bus / vn_lv_bus)
-            self.trafo_ratio_neutral = (tr.vn_hv_kv.to_numpy(float) / tr.vn_lv_kv.to_numpy(float)) / \
-                (vn_hv_bus / vn_lv_bus)
+            r, x, g, b, ratio, self.trafo_ratio_neutral = trafo_branch_values(
+                tr.vn_hv_kv.to_numpy(float), tr.vn_lv_kv.to_numpy(float), vn_hv_bus, vn_lv_bus,
+                tr.sn_mva.to_numpy(float), tr.vk_percent.to_numpy(float), tr.vkr_percent.to_numpy(float),
+                tr.pfe_kw.to_numpy(float), tr.i0_percent.to_numpy(float), steps, on_hv, on_lv,
+                tr.parallel.to_numpy(float), sn, self.trafo_model)
             self.trafo_tap_on_hv = on_hv
             self.trafo_tap_on_lv = on_lv
             shift = tr.shift_degree.to_numpy(float) if self.calculate_voltage_angles else np.zeros(nt)
             par = tr.parallel.to_numpy(float)
             sn_t = tr.sn_mva.to_numpy(float)
-            # short-circuit impedance, referred to the LV bus voltage
-            tap_lv = (vnl / vn_lv_bus) ** 2 * sn
-            z_sc = tr.vk_percent.to_numpy(float) / 100.0 / sn_t * tap_lv
-            r_sc = tr.vkr_percent.to_numpy(float) / 100.0 / sn_t * tap_lv
-            x_sc = np.sign(z_sc) * np.sqrt(z_sc ** 2 - r_sc ** 2)
-            r = r_sc / par
-            x = x_sc / par
-            # magnetising branch
-            base_r = vn_lv_bus ** 2 / sn
-            vnl_sq = tr.vn_lv_kv.to_numpy(float) ** 2
-            pfe = tr.pfe_kw.to_numpy(float) * 1e-3
-            g_m = pfe / vnl_sq * base_r
-            i0 = tr.i0_percent.to_numpy(float)
-            b_sq = (i0 / 100.0 * sn_t) ** 2 - pfe ** 2
-            b_sq[b_sq < 0] = 0.0
-            b_m = np.sqrt(b_sq) * base_r / vnl_sq * np.sign(i0)
-            y_sh = (g_m - 1j * b_m) / (vnl / tr.vn_lv_kv.to_numpy(float)) ** 2 * par
-            if self.trafo_model == "t":
-                nz = y_sh != 0
-                za = (r[nz] + 1j * x[nz]) / 2.0
-                zc = 1.0 / y_sh[nz]
-                zsum = za * za + 2.0 * za * zc
-                zab = zsum / zc
-                zbc = zsum / za
-                r = r.copy()
-                x = x.copy()
-                r[nz], x[nz] = zab.real, zab.imag
-                y_sh = y_sh.copy()
-                y_sh[nz] = 2.0 / zbc
             sl = slice(nl, nl + nt)
             br[sl, F_BUS] = self.trafo_h
             br[sl, T_BUS] = self.trafo_l
             br[sl, BR_R], br[sl, BR_X] = r, x
-            br[sl, BR_G], br[sl, BR_B] = y_sh.real, y_sh.imag
+            br[sl, BR_G], br[sl, BR_B] = g, b
             br[sl, TAP] = ratio
             br[sl, SHIFT] = shift
             df = tr.df.to_numpy(float)
@@ -366,6 +465,8 @@ class PpcBuilder:
             # trafo_loading='current': 100*max(i_hv*vn_hv, i_lv*vn_lv)*sqrt3/sn
             rate_f[sl] = tr.vn_hv_kv.to_numpy(float) / (vn_hv_bus * sn_t * par * df)
             rate_t[sl] = tr.vn_lv_kv.to_numpy(float) / (vn_lv_bus * sn_t * par * df)
+        if n3r:
+            self._trafo3w_table(net, br, rate_f, rate_t, nl + nt)
         if ni:
             # pandapower build_branch._calc_impedance_parameter [ext-mem]: per unit on the element's own
             # sn_mva, rescaled to the net's; no shunt part, ratio 1, no rating (res_impedance has no loading)
@@ -376,10 +477,52 @@ class PpcBuilder:
             if not (np.array_equal(rft, rtf) and np.array_equal(xft, xtf)):
                 raise NotImplementedError("net.impedance with rtf_pu != rft_pu or xtf_pu != xft_pu: the branch "
                                           "model of the kernels is symmetric (pandapower's BR_R_ASYM / BR_X_ASYM)")
-            sl = slice(nl + nt, nl + nt + ni)
+            sl = slice(nl + nt + n3r, nl + nt + n3r + ni)
             br[sl, F_BUS], br[sl, T_BUS] = self.imp_f, self.imp_t
             br[sl, BR_R], br[sl, BR_X] = rft, xft
         return br, rate_f, rate_t
+
+    def _trafo3w_table(self, net, br, rate_f, rate_t, first):
+        """Rows of the three 2-winding equivalents of every trafo3w (PANDAPOWER_ASSUMPTIONS 9-16)."""
+        t3 = net.trafo3w
+        n3 = len(t3)
+        vk_s, vkr_s, sn_s = trafo3w_star_parameters(t3)
+        vn_s = np.stack([t3[f"vn_{s}_kv"].to_numpy(float) for s in ("hv", "mv", "lv")])
+        zero = np.zeros(n3)
+        shift_s = np.stack([zero, t3.shift_mv_degree.to_numpy(float), t3.shift_lv_degree.to_numpy(float)])
+        side = t3.tap_side.to_numpy(object)
+        star = t3.tap_at_star_point.to_numpy(bool) if "tap_at_star_point" in t3 else np.zeros(n3, bool)
+        steps = np.nan_to_num(t3.tap_step_percent.to_numpy(float) * (t3.tap_pos.to_numpy(float) -
+                                                                    t3.tap_neutral.to_numpy(float)) / 100.0)
+        # winding w's branch carries the tap changer: at its outer end (hv row: hv side, mv / lv rows: lv side), at
+        # the star end with tap_at_star_point
+        self.trafo3w_tap_w = np.array([("hv", "mv", "lv").index(x) if x in ("hv", "mv", "lv") else -1 for x in side])
+        self.trafo3w_tap_at_lv = np.where(self.trafo3w_tap_w == 0, star, ~star)
+        ks = np.array([k for k, _ in self.trafo3w_rows], dtype=np.int64)
+        ws = np.array([w for _, w in self.trafo3w_rows], dtype=np.int64)
+        tapped = self.trafo3w_tap_w[ks] == ws
+        on_lv = tapped & self.trafo3w_tap_at_lv[ks]
+        on_hv = tapped & ~self.trafo3w_tap_at_lv[ks]
+        n = len(ks)
+        one = np.ones(n)
+        vn_f, vn_t = self.base_kv[self.trafo3w_f], self.base_kv[self.trafo3w_t]
+        hv_row = ws == 0
+        pfe = np.where(hv_row, t3.pfe_kw.to_numpy(float)[ks], 0.0)
+        i0 = np.where(hv_row, t3.i0_percent.to_numpy(float)[ks], 0.0)
+        r, x, g, b, ratio, self.trafo3w_ratio_neutral = trafo_branch_values(
+            vn_s[0, ks], vn_s[ws, ks], vn_f, vn_t, sn_s[ws, ks], vk_s[ws, ks], vkr_s[ws, ks], pfe, i0,
+            steps[ks], on_hv, on_lv, one, net.sn_mva, self.trafo_model)
+        sl = slice(first, first + n)
+        br[sl, F_BUS], br[sl, T_BUS] = self.trafo3w_f, self.trafo3w_t
+        br[sl, BR_R], br[sl, BR_X] = r, x
+        br[sl, BR_G], br[sl, BR_B] = g, b
+        br[sl, TAP] = ratio
+        br[sl, SHIFT] = shift_s[ws, ks] if self.calculate_voltage_angles else 0.0
+        br[sl, RATE_A] = sn_s[ws, ks]
+        # loading factors at the outer end only: vn_<side>_kv / (bus vn_kv * sn_<side>_mva)
+        rate = vn_s[ws, ks] / (np.where(hv_row, vn_f, vn_t) * sn_s[ws, ks])
+        rate_f[sl] = np.where(hv_row, rate, 0.0)
+        rate_t[sl] = np.where(hv_row, 0.0, rate)
 
     def build(self, net) -> Ppc:
         sn = net.sn_mva
@@ -468,7 +611,8 @@ class PpcBuilder:
                    trafo_branch=self.trafo_branch.copy(),
                    ext_grid_gen=ext_grid_gen, gen_gen=gen_gen,
                    rate_f=rate_f, rate_t=rate_t, init_vm_pu=init_vm,
-                   impedance_branch=self.impedance_branch.copy())
+                   impedance_branch=self.impedance_branch.copy(),
+                   trafo3w_branch=self.trafo3w_branch.copy())
 
 
 def build_ppc(net, **kwargs) -> Ppc:
