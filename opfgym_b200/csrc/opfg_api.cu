@@ -125,12 +125,11 @@ struct OpfgGrid {
     int act_ref_max = -1, obs_ref_max = -1;   // largest state cell the action / observation tables touch
     size_t smem_pf = 0, smem_score = 0;
     int n_blocks_sym = 0;          // blocks of the filled Jacobian (d.n_blocks counts storage slots)
-    int carveout_pct = -1;   // -1: leave the driver's default L1/shared split
     int envs_per_cta = 1;
     int stage_level = 0;           // k_pf_multi: 0 = hot tables staged, 1 = + warm, 2 = all (OPFG_HOT/WARM/COLD_TABLES)
     // lane-per-environment kernel: schedule, per-warp scratch in global memory, launch shape
     LaneSchedule lane;
-    int pf_kernel = 0;              // OpfgGridDesc.pf_kernel (after the OPFG_PF_KERNEL override)
+    int pf_kernel = 0;              // OpfgGridDesc.pf_kernel
     bool lanes_ok = false;          // tables built (the grid qualifies)
     double* lane_scratch = nullptr;
     size_t lane_warp_doubles = 0;   // scratch doubles per warp (32 lanes)
@@ -356,9 +355,8 @@ static ItemGrid item_grid(int64_t n_env, int n_items) {
     int w_log2 = 0;
     while ((1 << w_log2) < n_items && w_log2 < 8) ++w_log2;
     const int W = 1 << w_log2, epb = 256 / W;
-    static const int64_t y_cap = getenv("OPFG_ITEM_GRID_Y") ? atoll(getenv("OPFG_ITEM_GRID_Y")) : 8192;
     const int64_t groups = (n_env + epb - 1) / epb;
-    return {dim3((unsigned)((n_items + W - 1) / W), (unsigned)std::max<int64_t>(1, std::min<int64_t>(groups, y_cap))), w_log2};
+    return {dim3((unsigned)((n_items + W - 1) / W), (unsigned)std::max<int64_t>(1, std::min<int64_t>(groups, 8192))), w_log2};
 }
 #define OPFG_ITEM_LOOP(item, env, n_env_, w_log2)                                                   \
     const int item = (int)(blockIdx.x << (w_log2)) + (int)(threadIdx.x & ((1u << (w_log2)) - 1u));  \
@@ -533,21 +531,12 @@ __global__ void k_sample_profiles(uint64_t seed, uint64_t first_env, uint64_t st
                                                                noise_factor, noise_kind);
     }
 }
-template <int T>
-__global__ void __launch_bounds__(T) k_assemble(GridDev g, OpfgBatch B) {
-    Ctx<T> cx{(int)threadIdx.x, nullptr, 0};
-    const int64_t env = blockIdx.x;
-    env_assemble(g, cx, B.actions ? B.actions + env * g.n_act : nullptr, B.state + env * (int64_t)g.n_state,
-                 B.sbus ? B.sbus + env * (int64_t)g.nb * 2 : nullptr,
-                 B.yval ? B.yval + env * (int64_t)g.nnz_y * 2 : nullptr,
-                 B.bry ? B.bry + env * (int64_t)g.n_dyn * 8 : nullptr, B.absolute_actions != 0,
-                 B.vm ? B.vm + env * (int64_t)g.nb : nullptr);
-}
-// One warp per environment, W environments per CTA (lifts the 32-CTAs-per-SM limit on resident envs).
-// CAP: 0 = the compiler's default for 128-thread launches (56 / 62 registers); 3 = no occupancy target (70 / 72);
-// 1 / 2 / 4 = two-warp CTAs with at least 20 / 24 / 32 CTAs per SM (48 / 40 / 32 registers): both kernels wait on DRAM loads behind references, more resident warps = more loads in flight
-template <int CAP>
-__global__ void __launch_bounds__((CAP == 1 || CAP == 2 || CAP == 4) ? 64 : 128, CAP == 4 ? 32 : (CAP == 2 ? 24 : (CAP == 1 ? 20 : (CAP == 3 ? 1 : 0)))) k_assemble_warps(GridDev g, OpfgBatch B) {
+// One warp per environment, two environments per CTA (lifts the 32-CTAs-per-SM limit on resident envs).
+// Both kernels wait on DRAM loads behind references: more resident warps = more loads in flight.
+// k_assemble_warps keeps the compiler's default for 128-thread bounds (62 registers); k_score_warps asks for 24
+// two-warp CTAs per SM (40 registers).  Measured for k_score_warps (122-bus grid, 32 768 environments):
+// 56 registers 234 us, 48 -> 217, 40 -> 210, 70 -> 254.
+__global__ void __launch_bounds__(128) k_assemble_warps(GridDev g, OpfgBatch B) {
     const int64_t env = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (env >= B.n_env) return;
     Ctx<32> cx{(int)(threadIdx.x & 31), nullptr, 0};
@@ -557,8 +546,7 @@ __global__ void __launch_bounds__((CAP == 1 || CAP == 2 || CAP == 4) ? 64 : 128,
                  B.bry ? B.bry + env * (int64_t)g.n_dyn * 8 : nullptr, B.absolute_actions != 0,
                  B.vm ? B.vm + env * (int64_t)g.nb : nullptr);
 }
-template <int CAP>
-__global__ void __launch_bounds__((CAP == 1 || CAP == 2 || CAP == 4) ? 64 : 128, CAP == 4 ? 32 : (CAP == 2 ? 24 : (CAP == 1 ? 20 : (CAP == 3 ? 1 : 0)))) k_score_warps(GridDev g, OpfgBatch B, int env_doubles) {
+__global__ void __launch_bounds__(64, 24) k_score_warps(GridDev g, OpfgBatch B, int env_doubles) {
     extern __shared__ __align__(16) double sm[];
     const int64_t env = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (env >= B.n_env) return;
@@ -621,14 +609,14 @@ __global__ void __launch_bounds__(T) k_pf(GridDev g, OpfgBatch B) {
 // the schedule / Ybus tables (their reads are on the critical path of every level); each environment
 // group synchronises on its own named barrier and walks through its share of the batch.
 // Tables of the staged arena, in allocation order: the LU schedule and the Ybus index tables ("hot", always
-// staged), the Ybus values ("warm", read in every iteration) and the start-value / DC-factor / q-limit tables ("cold",
+// staged), the Ybus values ("warm", read in every iteration) and the start-value / q-limit tables ("cold",
 // read once per solve).  STAGE = 0 stages the hot part, 1 hot + warm, 2 everything -- whichever lets
 // the most environments share an SM.
 #define OPFG_HOT_TABLES(X)                                                                      \
-    X(bus_of_int) X(type_int) X(level_ptr) X(fill_ids) X(diag_mode) X(dp_ptr) X(dp_pack) X(dp_own) \
+    X(bus_of_int) X(type_int) X(level_ptr) X(fill_ids) X(dp_ptr) X(dp_pack) X(dp_own) \
     X(eg_ptr) X(eg_item) X(off_ptr) X(off_hdr) X(op_pack) X(up_ptr) X(up_pack) X(y_ptr) X(y_meta)
 #define OPFG_WARM_TABLES(X) X(y_val)
-#define OPFG_COLD_TABLES(X) X(vm0_int) X(va0_int) X(dc_val) X(dc_rhs0) X(qlim_bus) X(qlim_min) X(qlim_max)
+#define OPFG_COLD_TABLES(X) X(vm0_int) X(va0_int) X(qlim_bus) X(qlim_min) X(qlim_max)
 
 // The kernel receives a view of GridDev in which every staged table pointer holds its BYTE OFFSET in
 // the arena (staged_view below).  Adding the offset to the shared-memory base is one instruction and
@@ -671,9 +659,8 @@ __global__ void __launch_bounds__(BOUND, 1) k_pf_multi(GridDev g, OpfgBatch B, i
 }
 // Fused kernel for radial grids (opfg_core.h, env_pf_tree): persistent CTAs, E environments of T lanes
 // each (32 / T environments share a warp and run in lockstep), tables staged once per CTA.
-#define OPFG_TREE_TABLES(X) X(tr_bus_of_int) X(tr_level_ptr) X(tr_y_ptr) X(tr_parent) X(tr_type) X(tr_y_ent) X(tr_y_val) X(tr_vm0) X(tr_va0) \
-    X(tr_dc_inv) X(tr_dc_w) X(tr_dc_rhs0)
-template <int T, bool DYN, int MAX_THREADS = (T == 32 ? 768 : T * 32)>
+#define OPFG_TREE_TABLES(X) X(tr_bus_of_int) X(tr_level_ptr) X(tr_y_ptr) X(tr_parent) X(tr_type) X(tr_y_ent) X(tr_y_val) X(tr_vm0) X(tr_va0)
+template <int T, bool DYN, int MAX_THREADS>
 __global__ void __launch_bounds__(MAX_THREADS, 1) k_pf_tree(GridDev g, OpfgBatch B, int E, int env_doubles) {
     extern __shared__ __align__(16) double sm[];
     {
@@ -819,21 +806,18 @@ static GridDev staged_view(const GridDev& d, int stage) {
 // the 122-bus grid (B200, 32 768 environments): 8 lanes 1.27 ms, 16 lanes 1.00 ms, 32 lanes 1.26 ms --
 // the kernel is bound by the latency of its level chain, more lanes mean fewer rounds per level until
 // the idle lanes of the narrow levels cost more issue slots than the rounds save.
-static int tree_lanes() {
-    const int T = getenv("OPFG_TREE_LANES") ? atoi(getenv("OPFG_TREE_LANES")) : 16;
-    return (T == 8 || T == 16 || T == 32) ? T : 16;
-}
+constexpr int TREE_LANES = 16;
 
 // Radial grid with the dense DC pre-pass: the fused kernel (pf_kernel 0 = auto or 3 = radial)
 static bool use_tree(const OpfgGrid* G, const OpfgBatch* B) {
     (void)B;
     const GridDev& d = G->d;
-    return d.tr_ok && (G->pf_kernel == 0 || G->pf_kernel == 3) && (!d.init_dc || d.dc_pre || d.tr_dc);
+    return d.tr_ok && (G->pf_kernel == 0 || G->pf_kernel == 3) && (!d.init_dc || d.dc_pre);
 }
 
 // Which power-flow kernel a launch uses: the lane-per-environment kernel when its tables exist (row
 // patterns of at most 255 blocks, row buffer fits shared memory) and the DC start comes from the dense
-// pre-pass; else one CTA per environment.  OpfgGridDesc.pf_kernel / OPFG_PF_KERNEL=cta|lanes override.
+// pre-pass; else one CTA per environment.  Only OpfgGridDesc.pf_kernel = 2 selects it.
 static bool use_lanes(const OpfgGrid* G, const OpfgBatch* B) {
     (void)B;
     if (G->pf_kernel != 2) return false;
@@ -927,17 +911,15 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
 
         int T = desc->threads_per_env;
         Symbolic& s = G->sym;
-        // OPFG_PF_KERNEL=cta keeps the CTA-per-environment kernel (and its level-minimising ordering)
-        int pf_kernel = desc->pf_kernel;
-        if (const char* pfk = getenv("OPFG_PF_KERNEL"))
-            pf_kernel = !strcmp(pfk, "cta") ? 1 : (!strcmp(pfk, "lanes") ? 2 : (!strcmp(pfk, "radial") ? 3 : pf_kernel));
+        // pf_kernel 1 keeps the CTA-per-environment kernel (and its level-minimising ordering)
+        const int pf_kernel = desc->pf_kernel;
         G->pf_kernel = pf_kernel;
         const bool want_lanes = pf_kernel == 2;     // measured slower than the CTA kernels on B200 (DESIGN.md): opt-in
         analyse(nb, type, active, (desc->ordering == 0 && want_lanes) ? 3 : desc->ordering, T > 0 ? T : 32, s);
         if (desc->ordering == 0 && pf_kernel != 1 && pf_kernel != 2 && s.fill_ids.size() > 0) {
             // a radial grid has a fill-free (leaf-first) order, which is what the fused kernel needs
             Symbolic leaf_first;
-            analyse(nb, type, active, 1, T > 0 ? T : 32, leaf_first, tree_lanes());
+            analyse(nb, type, active, 1, T > 0 ? T : 32, leaf_first, TREE_LANES);
             bool forest = leaf_first.fill_ids.empty();
             for (int k = 0; k < leaf_first.n && forest; ++k) forest = leaf_first.up_ptr[k + 1] - leaf_first.up_ptr[k] <= 1;
             if (forest) s = leaf_first;
@@ -965,7 +947,6 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
         d.type_int = G->tab(type_int);
         d.level_ptr = G->tab(s.level_ptr); d.fill_ids = G->tab(s.fill_ids);
         if (s.n_blocks >= 65535 || nb >= 65535) { delete G; return fail("grid too large for 16-bit schedule ids (%d blocks)", s.n_blocks); }
-        const bool dc_prepass = getenv("OPFG_DC_PREPASS") ? atoi(getenv("OPFG_DC_PREPASS")) != 0 : true;
         {   // pack the schedule into 16-bit ids (halves the L1 footprint of the shared tables)
             // ---- storage slots of the blocks (meshed grids) ----
             // A block id names a 2x2 block of the filled Jacobian; the kernel addresses shared memory by SLOT.
@@ -981,9 +962,8 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
             std::vector<char> is_fill(s.n_blocks, 0);
             for (int f : s.fill_ids) is_fill[f] = 1;
             int n_slots = s.n_blocks;
-            // the DC start inside the kernel indexes its static factor by the packed ids: no sharing then
             const bool share_slots = (getenv("OPFG_SHARE_SLOTS") ? atoi(getenv("OPFG_SHARE_SLOTS")) != 0 : true) &&
-                                     !s.fill_ids.empty() && (dc_prepass || !desc->init_dc);
+                                     !s.fill_ids.empty();
             if (share_slots) {
                 const int NEVER = 1 << 30;
                 std::vector<int> level_of(s.n, 0), last(s.n_blocks, -1), born(s.n_blocks, -1);
@@ -1058,8 +1038,6 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
                 for (int e = s.y_ptr[r]; e < s.y_ptr[r + 1]; ++e)
                     ym[e] = U2{(uint32_t)s.y_col[e] | ((uint32_t)((s.y_blk[e] < 0 ? -1 : slot[s.y_blk[e]]) + 1) << 16), (uint32_t)r};
             d.nnz_y_nonref = s.y_ptr[s.n];
-            // per level: one lane per pivot, or eight lanes per pivot (component-parallel gather)
-            std::vector<unsigned char> mode(s.n_levels, 0);
             // Eager gather pays where few environments fit an SM and the phase latency is exposed
             // (meshed 372-bus grid: -7 %); with ten resident environments the kernel is bound by
             // shared-memory throughput and the extra partial-sum traffic costs 2 %.
@@ -1075,24 +1053,16 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
                 if (s.eg_count[i] > 0xffff) throw std::runtime_error("eager gather item with more than 65535 pairs");
                 eg[i] = U2{(uint32_t)s.eg_k[i] | ((uint32_t)s.eg_count[i] << 16), (uint32_t)s.eg_begin[i]};
             }
-            for (int l = 0; l < s.n_levels; ++l) {
-                int items = s.level_ptr[l + 1] - s.level_ptr[l] + s.eg_ptr[l + 1] - s.eg_ptr[l], maxp = 0;
-                for (int k = s.level_ptr[l]; k < s.level_ptr[l + 1]; ++k) maxp = std::max(maxp, s.dp_ptr[k + 1] - s.dp_own[k]);
-                for (int i = s.eg_ptr[l]; i < s.eg_ptr[l + 1]; ++i) maxp = std::max(maxp, s.eg_count[i]);
-                if (getenv("OPFG_DEBUG_SCHEDULE"))
+            if (getenv("OPFG_DEBUG_SCHEDULE"))
+                for (int l = 0; l < s.n_levels; ++l) {
+                    int maxp = 0;
+                    for (int k = s.level_ptr[l]; k < s.level_ptr[l + 1]; ++k) maxp = std::max(maxp, s.dp_ptr[k + 1] - s.dp_own[k]);
+                    for (int i = s.eg_ptr[l]; i < s.eg_ptr[l + 1]; ++i) maxp = std::max(maxp, s.eg_count[i]);
                     fprintf(stderr, "level %d: own %d eager %d max pairs %d (own max %d) off items %d\n", l,
                             s.level_ptr[l + 1] - s.level_ptr[l], s.eg_ptr[l + 1] - s.eg_ptr[l], maxp,
                             [&] { int m = 0; for (int k = s.level_ptr[l]; k < s.level_ptr[l + 1]; ++k) m = std::max(m, s.dp_ptr[k + 1] - s.dp_ptr[k]); return m; }(),
                             s.off_ptr[l + 1] - s.off_ptr[l]);
-                const double narrow = std::ceil(items / (double)T) * (45.0 + 30.0 * maxp);
-                const double wide = std::ceil(items * 8 / (double)T) * (75.0 + 12.0 * maxp);
-                // Measured on the grids that still take this kernel (round 2, final code): one lane per pivot everywhere
-                // beats the model's choice (EcoDispatch 2.785 vs 2.807 ms/step, LoadShedding + ties 13.85 vs 13.60 M env
-                // steps/s; eight lanes per pivot everywhere: 3.96 ms / 11.0 M).  OPFG_DIAG_MODE=model restores the model.
-                const char* dm = getenv("OPFG_DIAG_MODE");
-                mode[l] = !dm ? 0 : (strcmp(dm, "model") == 0 ? (wide < narrow ? 1 : 0) : (atoi(dm) ? 1 : 0));
-            }
-            d.diag_mode = G->tab(mode);
+                }
             d.dp_ptr = G->tab(s.dp_ptr); d.dp_pack = G->tab(dp);
             d.dp_own = G->tab(s.dp_own); d.eg_ptr = G->tab(s.eg_ptr); d.eg_item = G->tab(eg);
             d.off_ptr = G->tab(s.off_ptr); d.off_hdr = G->tab(hdr); d.op_pack = G->tab(op);
@@ -1109,7 +1079,7 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
         double* y_val = G->tab(std::vector<double>(2 * s.y_col.size(), 0.0));
         d.y_val = y_val;
         d.tab_warm_bytes = (int)((G->tab_used + 15) & ~size_t(15));   // tables read in every iteration end here
-        d.vm0_int = G->tab(vm0); d.va0_int = G->tab(va0);              // start values, DC factor, q-limits: once per solve
+        d.vm0_int = G->tab(vm0); d.va0_int = G->tab(va0);              // start values, q-limits: once per solve
 
         // DC start: scalar factor of B' on the same schedule + constant part of its rhs
         std::vector<double> dc_val, dc_rhs0(s.n, 0.0);
@@ -1130,11 +1100,11 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
         for (int k = 0; k < s.n; ++k) dc_rhs0[k] -= ysh[2 * s.bus_of_int[k]];
         d.dc_pre = 0; d.dc_binv_t = nullptr; d.dc_theta0 = nullptr; d.dc_ld = 0;
         // Dense pre-pass for the DC start: theta = B'^-1 (P + rhs0) for ALL environments as one FP64
-        // GEMM (k_dc_start).  Inside the persistent kernel the same solve is 2 x levels barrier phases
+        // GEMM (k_dc_start).  Inside the persistent kernel the same solve was 2 x levels barrier phases
         // of dependent scalar work: 17 % of the kernel on the 372-bus grid (4.47 -> 3.82 ms with the
         // pre-pass), 11 % on the 122-bus grid (0.14 ms in the kernel against 0.08 ms for the GEMM).
-        // B'^-1 is built column by column with the factor the kernel would use.
-        if (desc->init_dc && s.n > 0 && dc_prepass) {
+        // B'^-1 is built column by column from the sparse factor of B' on the power-flow schedule.
+        if (desc->init_dc && s.n > 0) {
             const int n = s.n, ld = (n + 63) / 64 * 64, kp = (nb + 15) / 16 * 16;   // rows: ppc bus order (coalesced P reads)
             std::vector<double> binv_t((size_t)kp * ld, 0.0), x(n), theta0(n, 0.0);
             auto solve = [&](std::vector<double>& v) {
@@ -1160,13 +1130,6 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
             theta0 = dc_rhs0;
             solve(theta0);
             d.dc_binv_t = G->up(binv_t); d.dc_theta0 = G->up(theta0); d.dc_ld = ld; d.dc_pre = 1;
-        }
-        if (d.dc_pre) {
-            // the kernel never touches the sparse DC factor then: it stays out of the staged arena
-            // (4.6 KB on the 122-bus grid -- exactly what an 11th environment per SM was missing)
-            d.dc_val = d.dc_rhs0 = reinterpret_cast<const double*>(G->tab_base);
-        } else {
-            d.dc_val = G->tab(dc_val); d.dc_rhs0 = G->tab(dc_rhs0);
         }
         std::vector<int> lane_qb;
         std::vector<double> lane_qmn, lane_qmx;
@@ -1253,40 +1216,24 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
                 d.tr_bus_of_int = G->tab(s.bus_of_int); d.tr_level_ptr = G->tab(s.level_ptr);
                 d.tr_y_ptr = G->tab(s.y_ptr); d.tr_parent = G->tab(parent);
                 d.tr_y_ent = G->tab(col); d.tr_type = G->tab(type_int);
-                // DC start inside the kernel: 1 / d_k and W_k = B'_kp / d_k of the leaf-first factor of B'
-                d.tr_dc = 0; d.tr_dc_inv = d.tr_dc_w = d.tr_dc_rhs0 = d.tr_vm0;
-                // opt-in (OPFG_TREE_DC=1): measured SLOWER on B200 than the GEMM pre-pass -- 36 more dependent phases of
-                // index -> index -> value shared-memory chains cost 110 us per 32 768 environments, the GEMM 83 us
-                const bool dc_in_tree = getenv("OPFG_TREE_DC") ? atoi(getenv("OPFG_TREE_DC")) != 0 : false;
-                if (desc->init_dc && dc_ok && dc_in_tree) {
-                    std::vector<double> inv(s.n), w(s.n, 0.0);
-                    for (int k = 0; k < s.n; ++k) {
-                        inv[k] = dc_val[k];
-                        if (s.up_ptr[k + 1] > s.up_ptr[k]) w[k] = dc_val[s.up_w[s.up_ptr[k]]];
-                    }
-                    d.tr_dc_inv = G->tab(inv); d.tr_dc_w = G->tab(w); d.tr_dc_rhs0 = G->tab(dc_rhs0);
-                    d.tr_dc = 1;
-                }
                 d.tab4_bytes = (int)((G->tab_used + 15) & ~size_t(15));
                 G->tab_base = keep_base; G->tab_cap = keep_cap; G->tab_used = keep_used;
                 d.tr_ok = 1;
             }
         }
-        if (const char* cv = getenv("OPFG_CARVEOUT")) G->carveout_pct = atoi(cv);
         G->smem_pf = (pf_smem_doubles(d.n_blocks, s.n, nb, T, d.n_qlim) * sizeof(double) + 31) & ~size_t(31);
         {   // environments per CTA: stage the tables in shared memory when several environments share them
             const size_t budget = 227 * 1024;
             const int cap = std::min(15, 768 / T);    // named barriers 1..15; k_pf_multi is bounded to 768 threads
             // stage everything if at least two environments still fit; else the tables read in every
             // iteration; else only the LU schedule.  (Measured on the 122-bus grid: an 11th environment
-            // bought by leaving the start-value / DC tables in global memory is a net loss, 1.46 vs 1.41 ms.)
+            // bought by leaving the start-value tables in global memory is a net loss, 1.46 vs 1.41 ms.)
             auto fit = [&](int bytes) { return (size_t)bytes < budget ? std::min((int)((budget - bytes) / G->smem_pf), cap) : 0; };
             const int sizes[3] = {d.tab_hot_bytes, d.tab_warm_bytes, d.tab_bytes};
             int level = fit(sizes[2]) >= 2 ? 2 : ((fit(sizes[1]) >= 2 && (size_t)sizes[1] * 3 <= budget) ? 1 : 0);
             // with two environments per SM the kernel is latency-bound on 8 warps: a third environment is worth
             // more than staged Ybus tables (372-bus grid, shared slots: 3 x 61 KB + the 34 KB LU schedule)
-            static const bool prefer_envs = getenv("OPFG_PREFER_ENVS") ? atoi(getenv("OPFG_PREFER_ENVS")) != 0 : true;
-            if (prefer_envs && fit(sizes[level]) <= 2)
+            if (fit(sizes[level]) <= 2)
                 for (int lv = level - 1; lv >= 0; --lv)
                     if (fit(sizes[lv]) > fit(sizes[level])) level = lv;
             if (const char* sv = getenv("OPFG_STAGE")) level = std::max(0, std::min(2, atoi(sv)));
@@ -1323,10 +1270,10 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
             cudaMemcpy(const_cast<double*>(d.tr_y_val), y_val, ybytes, cudaMemcpyDeviceToDevice);
             // lanes per environment: narrow levels (one pivot per feeder) leave wider groups idle; the
             // environments that fit shared memory decide how many warps an SM gets
-            const int T = tree_lanes();
+            constexpr int T = TREE_LANES;
             const size_t budget = 227 * 1024, per_env = G->tree_env_doubles * sizeof(double);
             int E = (size_t)d.tab4_bytes < budget ? (int)((budget - d.tab4_bytes) / per_env) : 0;
-            E = std::min(E, T == 32 ? 24 : 32);          // the kernel's launch bounds
+            E = std::min(E, 32);                       // the kernel's launch bounds (512 threads)
             if (const char* ev = getenv("OPFG_TREE_ENVS")) E = std::min(E, atoi(ev));
             E -= E % (32 / T);                         // whole warps
             if (E < 32 / T) d.tr_ok = 0;
@@ -1353,10 +1300,8 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
             // launch shape: W warps per CTA, one CTA per SM; shared memory = tables (if they fit) + W row buffers
             const size_t rb_bytes = sizeof(double) * 4 * (size_t)d.ln_max_row * 32;
             const size_t budget = 227 * 1024;
-            int W = getenv("OPFG_LANE_WARPS") ? atoi(getenv("OPFG_LANE_WARPS")) : 12;
-            W = std::max(1, std::min(W, 16));
-            bool staged = (size_t)d.tab3_bytes + rb_bytes <= budget;
-            if (const char* sv = getenv("OPFG_LANE_STAGE")) staged = staged && atoi(sv) != 0;
+            int W = 12;
+            const bool staged = (size_t)d.tab3_bytes + rb_bytes <= budget;
             const size_t tabs = staged ? (size_t)d.tab3_bytes : 0;
             while (W > 1 && tabs + W * rb_bytes > budget) --W;
             if (tabs + W * rb_bytes > budget) G->lanes_ok = false;     // one row buffer does not fit: CTA kernel
@@ -1645,7 +1590,6 @@ int opfg_set_scoring(OpfgGrid* G, const OpfgScoringDesc* sc) {
             G->obs_ref_max = std::max(G->obs_ref_max, sc->obs_ref[i]);
         d.obs_ptr = sc->obs_ptr ? G->tab2(sc->obs_ptr, sc->n_obs + 1) : nullptr;
         d.n_obs_runs = 0; d.obs_runs = nullptr;
-        d.score_prefetch = getenv("OPFG_SCORE_PREFETCH") ? atoi(getenv("OPFG_SCORE_PREFETCH")) : 2;
         if (!sc->obs_ptr && sc->n_obs > 0) {      // runs of consecutive state cells (observation keys are whole columns)
             std::vector<int> runs;
             bool ok = true;
@@ -1656,7 +1600,7 @@ int opfg_set_scoring(OpfgGrid* G, const OpfgScoringDesc* sc) {
                 runs.insert(runs.end(), {sc->obs_ref[i], i, j - i});
                 i = j;
             }
-            if (ok && runs.size() / 3 <= 64 && (int)(runs.size() / 3) * 8 <= sc->n_obs && !getenv("OPFG_NO_OBS_RUNS")) {
+            if (ok && runs.size() / 3 <= 64 && (int)(runs.size() / 3) * 8 <= sc->n_obs) {
                 d.obs_runs = G->up(runs);
                 d.n_obs_runs = (int)(runs.size() / 3);
             }
@@ -1833,12 +1777,7 @@ int opfg_assemble(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
                      B->bry ? B->bry + env * (int64_t)G->d.n_dyn * 8 : nullptr, B->absolute_actions != 0,
                      B->vm ? B->vm + env * (int64_t)G->d.nb : nullptr);
 #else
-    {
-        static int warps = getenv("OPFG_AUX_WARPS") ? atoi(getenv("OPFG_AUX_WARPS")) : 2;
-        static int cap = getenv("OPFG_ASSEMBLE_CAP") ? atoi(getenv("OPFG_ASSEMBLE_CAP")) : 0;
-        void (*fn)(GridDev, OpfgBatch) = (warps == 2 && cap == 2) ? k_assemble_warps<2> : ((warps == 2 && cap == 1) ? k_assemble_warps<1> : (cap == 3 ? k_assemble_warps<3> : k_assemble_warps<0>));
-        fn<<<(unsigned)((B->n_env + warps - 1) / warps), 32 * warps, 0, (cudaStream_t)stream>>>(G->d, *B);
-    }
+    k_assemble_warps<<<(unsigned)((B->n_env + 1) / 2), 64, 0, (cudaStream_t)stream>>>(G->d, *B);
     ++g_launches;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail("assemble launch: %s", cudaGetErrorString(e));
@@ -1854,7 +1793,7 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
     (void)stream;
     Ctx<1> cx;
     std::vector<double> sm(pf_smem_doubles(G->d.n_blocks, G->d.n, G->d.nb, 32, G->d.n_qlim));
-    if (G->d.dc_pre && !(use_tree(G, B) && G->d.tr_dc)) {   // the dense DC pre-pass, as a plain loop (the radial kernel has its own DC start)
+    if (G->d.dc_pre) {   // the dense DC pre-pass, as a plain loop
         const GridDev& d = G->d;
         for (int64_t env = 0; env < B->n_env; ++env)
             for (int i = 0; i < d.n; ++i) {
@@ -1895,7 +1834,7 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
                      (G->d.n_dyn > 0 && B->yval) ? B->yval + env * (int64_t)G->d.nnz_y * 2 : nullptr, B->vm + env * (int64_t)G->d.nb,
                      B->va + env * (int64_t)G->d.nb, B->converged + env, B->iterations + env);
 #else
-    if (G->d.dc_pre && !(use_tree(G, B) && G->d.tr_dc)) {   // the radial kernel has its own DC start
+    if (G->d.dc_pre) {
         ensure_dynamic_smem(k_dc_start, DC_SMEM);
         k_dc_start<<<dim3((unsigned)((B->n_env + DC_ENVS - 1) / DC_ENVS), (unsigned)((G->d.n + 63) / 64)), 256, DC_SMEM, (cudaStream_t)stream>>>(G->d, *B);
         ++g_launches;
@@ -1903,22 +1842,20 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
     if (use_tree(G, B)) {
         OpfgGrid* Gm = const_cast<OpfgGrid*>(G);
         const bool dyn = G->d.n_dyn > 0 && B->yval;
-        // the last two: 16 lanes x at most 24 environments with the register cap of 384 threads (155 instead of 128)
-        void (*fns[8])(GridDev, OpfgBatch, int, int) = {k_pf_tree<8, false>, k_pf_tree<16, false>, k_pf_tree<32, false>,
-                                                        k_pf_tree<8, true>, k_pf_tree<16, true>, k_pf_tree<32, true>,
-                                                        k_pf_tree<16, false, 384>, k_pf_tree<16, true, 384>};
+        constexpr int T = TREE_LANES;
+        // at most 24 environments take the register cap of 384 threads (155 instead of 128 registers).  Measured on
+        // B200 (122-bus grid, 32 768 environments): 0.80 instead of 0.90 ms -- under the 128-register cap the
+        // staged-table base addresses were recomputed at their use sites
+        void (*fns[4])(GridDev, OpfgBatch, int, int) = {k_pf_tree<T, false, 512>, k_pf_tree<T, true, 512>,
+                                                        k_pf_tree<T, false, 384>, k_pf_tree<T, true, 384>};
         if (!Gm->tree_attr_set) {      // per grid, hence per device
             for (auto* f : fns) cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
             Gm->tree_attr_set = true;
         }
-        const int T = G->tree_T, E = G->tree_E;
+        const int E = G->tree_E;
         const int64_t groups = (B->n_env + E - 1) / E;
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(groups, G->n_sm));
-        auto* fn = fns[(T == 8 ? 0 : (T == 16 ? 1 : 2)) + (dyn ? 3 : 0)];
-        // measured on B200 (122-bus grid, 32 768 environments): 0.80 instead of 0.90 ms -- under the 128-register cap
-        // the staged-table base addresses were recomputed at their use sites
-        static const bool wide_regs = getenv("OPFG_TREE_WIDE_REGS") ? atoi(getenv("OPFG_TREE_WIDE_REGS")) != 0 : true;
-        if (wide_regs && T == 16 && E <= 24) fn = fns[dyn ? 7 : 6];
+        auto* fn = fns[(E <= 24 ? 2 : 0) + (dyn ? 1 : 0)];
         fn<<<grid, T * E, G->tree_smem, (cudaStream_t)stream>>>(tree_view(G->d), *B, E, (int)G->tree_env_doubles);
         ++g_launches;
         cudaError_t e = cudaGetLastError();
@@ -1948,13 +1885,6 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
     const size_t smem = G->smem_pf;
     OPFG_DISPATCH_T(G->d.threads, {
         ensure_dynamic_smem(k_pf<TT>, smem);
-        static int carve_set = -1;
-        if (G->carveout_pct >= 0 && carve_set != G->carveout_pct) {
-            // leave part of the unified L1/shared array to L1: the shared schedule tables must stay
-            // L1-resident, otherwise every table read is an L2 round trip on the critical path
-            cudaFuncSetAttribute(k_pf<TT>, cudaFuncAttributePreferredSharedMemoryCarveout, G->carveout_pct);
-            carve_set = G->carveout_pct;
-        }
         if (G->envs_per_cta > 1) {
             const int E = G->envs_per_cta;
             const size_t smem_multi = G->d.tab_staged_bytes + (size_t)E * smem;
@@ -1965,8 +1895,7 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
             const GridDev view = staged_view(G->d, stage);
             const int env_doubles = (int)(smem / 8);
             void (*fn)(GridDev, OpfgBatch, int, int) = nullptr;
-            static const bool roomy = getenv("OPFG_MULTI_ROOMY") ? atoi(getenv("OPFG_MULTI_ROOMY")) != 0 : true;
-            const int bound = !roomy ? 768 : (TT * E <= 256 ? 256 : (TT * E <= 384 ? 384 : 768));   // 384 = three HV environments of 128 threads: 168 registers
+            const int bound = TT * E <= 256 ? 256 : (TT * E <= 384 ? 384 : 768);   // 384 = three HV environments of 128 threads: 168 registers
             switch (stage | ((G->d.n_dyn > 0 && B->yval) ? 4 : 0)) {
                 case 0: fn = pick_multi<TT, 0>(bound); break;
                 case 1: fn = pick_multi<TT, 1>(bound); break;
@@ -2003,21 +1932,17 @@ int opfg_score(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
                   B->state + env * (int64_t)G->d.n_state);
 #else
     const size_t smem = score_smem_doubles(G->d.nb, G->d.nbr, G->score_threads) * sizeof(double);
-    OPFG_DISPATCH_T(G->score_threads, {
-        ensure_dynamic_smem(k_score<TT>, smem);
-        if (TT == 32) {
-            static int warps = getenv("OPFG_AUX_WARPS") ? atoi(getenv("OPFG_AUX_WARPS")) : 2;
-            const size_t per_env = (smem + 15) & ~size_t(15);
-            // measured (122-bus grid, 32 768 environments): 56 registers 234 us, 48 -> 217, 40 -> 210, 70 -> 254
-            static int cap = getenv("OPFG_SCORE_CAP") ? atoi(getenv("OPFG_SCORE_CAP")) : 2;
-            void (*fn)(GridDev, OpfgBatch, int) = (warps == 2 && cap == 4) ? k_score_warps<4> : (warps == 2 && cap == 2) ? k_score_warps<2> : ((warps == 2 && cap == 1) ? k_score_warps<1> : (cap == 3 ? k_score_warps<3> : k_score_warps<0>));
-            ensure_dynamic_smem(fn, per_env * warps);
-            fn<<<(unsigned)((B->n_env + warps - 1) / warps), 32 * warps, per_env * warps, (cudaStream_t)stream>>>(
-                G->d, *B, (int)(per_env / 8));
-        } else {
-            k_score<TT><<<(unsigned)B->n_env, TT, smem, (cudaStream_t)stream>>>(G->d, *B);
-        }
-    });
+    if (G->score_threads == 32) {
+        const size_t per_env = (smem + 15) & ~size_t(15);
+        ensure_dynamic_smem(k_score_warps, per_env * 2);
+        k_score_warps<<<(unsigned)((B->n_env + 1) / 2), 64, per_env * 2, (cudaStream_t)stream>>>(G->d, *B, (int)(per_env / 8));
+    } else {
+        const int T = G->score_threads;
+        void (*fn)(GridDev, OpfgBatch) = T == 64 ? k_score<64> : (T == 128 ? k_score<128> : (T == 256 ? k_score<256> : nullptr));
+        if (!fn) return fail("unsupported threads_per_env %d", T);
+        ensure_dynamic_smem(fn, smem);
+        fn<<<(unsigned)B->n_env, T, smem, (cudaStream_t)stream>>>(G->d, *B);
+    }
     ++g_launches;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail("score launch: %s", cudaGetErrorString(e));

@@ -42,7 +42,6 @@ struct GridDev {
     const double* va0_int;             // start angle (rad); ref buses keep it
     // schedule
     const int* level_ptr;
-    const unsigned char* diag_mode;    // [n_levels] 0: one lane per pivot, 1: eight lanes per pivot
     const int* fill_ids;
     // packed 16-bit block / pivot ids (n_blocks, nb < 65536 is checked at grid creation)
     const int* dp_ptr;                 // [n+1] pair ranges of the diagonal items
@@ -89,9 +88,6 @@ struct GridDev {
     int isl;
     const unsigned char* dyn_crit;     // [n_dyn] 1: the branch is a spanning-tree edge
     const int *isl_ptr, *isl_adj, *isl_br;   // CSR by ppc bus over the branches that can be in service: neighbour bus, branch row
-    // DC start
-    const double* dc_val;              // [n_blocks] scalar factor on the same schedule
-    const double* dc_rhs0;             // [n]
     // ---- assembly (kernel 1) ----
     int n_state, n_const, n_act, n_inj;
     double act_diff_step;
@@ -130,7 +126,6 @@ struct GridDev {
     int n_obs;
     const int* obs_ref;
     const int* obs_ptr;      // nullptr: one ref per observation
-    int score_prefetch;      // kernel 5: 0 no prefetch of the state row, 1 whole row, 2 observation runs only
     int n_obs_runs;          // > 0: the observation is a few runs of consecutive state cells
     const int* obs_runs;     // [n_obs_runs][3] first state cell, first observation entry, length
     // ---- lane-per-environment power flow (row-wise schedule, symbolic.hpp LaneSchedule) ----
@@ -157,10 +152,6 @@ struct GridDev {
     const unsigned char* tr_type;
     const uint32_t* tr_y_ent;          // per Ybus entry: column | kind << 16 (0 other, 1 child, 2 parent)
     const double *tr_y_val, *tr_vm0, *tr_va0;
-    // DC start inside the radial kernel (B' of a tree: one upward and one downward sweep of scalars):
-    // y_k = P_k + rhs0_k - sum_children W_c y_c;  theta_k = y_k / d_k - W_k theta_parent,  W_k = B'_kp / d_k
-    int tr_dc;
-    const double *tr_dc_inv, *tr_dc_w, *tr_dc_rhs0;
     const char* tab4_base;
     int tab4_bytes;
     const char* tab_base;              // contiguous arena holding the power-flow tables
@@ -213,15 +204,6 @@ struct Ctx {
         }
         return bad > 0 ? NAN : v;
     }
-    __device__ __forceinline__ bool wide_diag(unsigned char mode) const { return mode != 0; }
-    // values of lanes 0..5 of every aligned group of 8 lanes, broadcast to the whole group
-    __device__ __forceinline__ void gather8(double v, double& a, double& b, double& c, double& d,
-                                            double& y0, double& y1) const {
-        const int base = (tid & 31) & ~7;
-        a = __shfl_sync(0xffffffffu, v, base);      b = __shfl_sync(0xffffffffu, v, base + 1);
-        c = __shfl_sync(0xffffffffu, v, base + 2);  d = __shfl_sync(0xffffffffu, v, base + 3);
-        y0 = __shfl_sync(0xffffffffu, v, base + 4); y1 = __shfl_sync(0xffffffffu, v, base + 5);
-    }
     __device__ __forceinline__ double block_sum(double v) const {
         v = warp_sum(v);
         if (T > 32) {
@@ -244,8 +226,6 @@ struct Ctx {
     int bar_id = 0;
     int nthreads() const { return 1; }
     void sync() const {}
-    bool wide_diag(unsigned char) const { return false; }   // host walk: always one "lane" per pivot
-    void gather8(double, double&, double&, double&, double&, double&, double&) const {}
     double block_max(double v) const { return v; }
     double block_sum(double v) const { return v; }
 };
@@ -612,7 +592,7 @@ OPFG_HD void lu_eager_item(const GridDev& g, const PfSmem& s, U2 it) {
     st2(s.lu1 + 2 * k, r1.x, r1.y);
     st2(s.rhs + 2 * k, y.x, y.y);
 }
-// (a) one lane per pivot
+// one lane per pivot
 OPFG_HD void lu_diag_item(const GridDev& g, const PfSmem& s, int k) {
     D2 r0 = ld2(s.lu + 2 * k), r1 = ld2(s.lu1 + 2 * k), y = ld2(s.rhs + 2 * k);
     lu_gather_pairs(g, s, g.dp_own[k], g.dp_ptr[k + 1], r0, r1, y);
@@ -621,39 +601,6 @@ OPFG_HD void lu_diag_item(const GridDev& g, const PfSmem& s, int k) {
     st2(s.lu + 2 * k, ia, ib);
     st2(s.lu1 + 2 * k, ic, id_);
     st2(s.rhs + 2 * k, fma(ia, y.x, ib * y.y), fma(ic, y.x, id_ * y.y));
-}
-
-// (b) eight lanes per pivot: lane `sub` < 4 owns element (sub>>1, sub&1) of the block,
-// lanes 4 and 5 own y_0 and y_1 (short, independent gather chains instead of one long one)
-OPFG_HD double* lu_component_cell(const PfSmem& s, int k, int sub) {
-    const int r = sub < 4 ? (sub >> 1) : (sub - 4);
-    return sub < 4 ? (r ? s.lu1 : s.lu) + 2 * k + (sub & 1) : s.rhs + 2 * k + r;
-}
-OPFG_HD double lu_diag_component(const GridDev& g, const PfSmem& s, int k, int sub, int p, int pe) {
-    const int r = sub < 4 ? (sub >> 1) : (sub - 4);
-    double acc = *lu_component_cell(s, k, sub);
-#pragma unroll 4
-    for (; p < pe; ++p) {
-        const U2 id = g.dp_pack[p];
-        const D2 l = ld2((r ? s.lu1 : s.lu) + 2 * (id.x & 0xffffu));
-        double wa, wb;
-        if (sub < 4) { const int wi = 2 * (int)(id.x >> 16) + (sub & 1); wa = s.lu[wi]; wb = s.lu1[wi]; }
-        else { const D2 t = ld2(s.rhs + 2 * id.y); wa = t.x; wb = t.y; }
-        acc = fma(-l.y, wb, fma(-l.x, wa, acc));
-    }
-    return acc;
-}
-
-OPFG_HD void lu_diag_finish(const PfSmem& s, int k, int sub, double a, double b, double c, double d,
-                            double y0, double y1) {
-    const double r = 1.0 / fma(a, d, -(b * c));
-    const double ia = d * r, ib = -b * r, ic = -c * r, id_ = a * r;
-    if (sub == 0) s.lu[2 * k] = ia;
-    else if (sub == 1) s.lu[2 * k + 1] = ib;
-    else if (sub == 2) s.lu1[2 * k] = ic;
-    else if (sub == 3) s.lu1[2 * k + 1] = id_;
-    else if (sub == 4) s.rhs[2 * k] = fma(ia, y0, ib * y1);
-    else if (sub == 5) s.rhs[2 * k + 1] = fma(ic, y0, id_ * y1);
 }
 
 // An off-diagonal item in two parts.  The GATHER (target -= sum L~ W over pairs from lower levels) depends on
@@ -709,7 +656,8 @@ OPFG_HD void bwd_item(const GridDev& g, const PfSmem& s, int k) {
     st2(s.rhs + 2 * k, x.x, x.y);
 }
 
-// One environment: DC start, Newton-Raphson to tolerance, write |V|, angle, flag.
+// One environment: start values (the DC start comes from the dense pre-pass), Newton-Raphson to tolerance,
+// write |V|, angle, flag.
 // Mirrors pandapower newtonpf control flow (SURVEY.md App. B.4): convergence is
 // tested before the first iteration; at most max_iter linear solves.
 template <class C>
@@ -731,40 +679,14 @@ OPFG_HD void env_pf_solve(const GridDev& g, const C& cx, double* smem, const dou
         cx.sync();
     }
 
-    if (g.init_dc && !g.dc_pre) {   // pandapower init='dc': B' theta = P on the shared, pre-factorised B'
-        for (int k = cx.tid; k < n; k += T) s.rhs[k] = sbus[2 * g.bus_of_int[k]] + g.dc_rhs0[k];
-        cx.sync();
-        for (int l = 0; l < g.n_levels; ++l) {
-            for (int k = g.level_ptr[l] + cx.tid; k < g.level_ptr[l + 1]; k += T) {
-                double y = s.rhs[k];
-                for (int p = g.dp_ptr[k]; p < g.dp_ptr[k + 1]; ++p) {
-                    const U2 pr = g.dp_pack[p];
-                    y = fma(-g.dc_val[pr.x & 0xffffu], s.rhs[pr.y], y);
-                }
-                s.rhs[k] = y * g.dc_val[k];
-            }
-            cx.sync();
-        }
-        for (int l = g.n_levels - 1; l >= 0; --l) {
-            for (int k = g.level_ptr[l] + cx.tid; k < g.level_ptr[l + 1]; k += T) {
-                double x = s.rhs[k];
-                for (int p = g.up_ptr[k]; p < g.up_ptr[k + 1]; ++p) {
-                    const uint32_t pr = g.up_pack[p];
-                    x = fma(-g.dc_val[pr & 0xffffu], s.rhs[pr >> 16], x);
-                }
-                s.rhs[k] = x;
-            }
-            cx.sync();
-        }
-    }
-    OPFG_TICK(0);   // DC start
+    OPFG_TICK(0);   // q-limit set-up
     // |V| and angle are touched only by their owner lane, once per iteration: they live in the
     // output buffers (L2) instead of shared memory, which buys one more resident environment per SM
     for (int i = cx.tid; i < nb; i += T) {
         const int bus = g.bus_of_int[i];
         const double vm = g.vm_from_state ? vm_out[bus] : g.vm0_int[i];
         const bool dead = g.isl && vm == 0.0;                 // kernel 1 found the bus cut off from every slack
-        const double va = dead ? 0.0 : ((g.init_dc && i < n) ? (g.dc_pre ? va_out[bus] : s.rhs[i]) : g.va0_int[i]);
+        const double va = dead ? 0.0 : ((g.init_dc && i < n) ? va_out[bus] : g.va0_int[i]);   // DC start: written by the dense pre-pass
         double sn, cs;
         sincos(va, &sn, &cs);
         vm_out[bus] = vm; va_out[bus] = va; s.ivm[i] = dead ? 0.0 : 1.0 / vm;
@@ -806,25 +728,9 @@ OPFG_HD void env_pf_solve(const GridDev& g, const C& cx, double* smem, const dou
         for (int l = 0; l < g.n_levels; ++l) {
             const int lb = g.level_ptr[l], le = g.level_ptr[l + 1];
             const int n_own = le - lb, eb = g.eg_ptr[l], n_items = n_own + g.eg_ptr[l + 1] - eb;
-            if (cx.wide_diag(g.diag_mode[l])) {
-                const int sub = cx.tid & 7, grp = cx.tid >> 3, ngrp = T >> 3;
-                for (int base = 0; base < n_items; base += ngrp) {   // uniform trip count per warp
-                    const int idx = base + grp;
-                    const bool own = idx < n_own && sub < 6, eager = idx >= n_own && idx < n_items && sub < 6;
-                    int k = lb + idx, p = 0, pe = 0;
-                    if (own) { p = g.dp_own[k]; pe = g.dp_ptr[k + 1]; }
-                    else if (eager) { const U2 it = g.eg_item[eb + idx - n_own]; k = (int)(it.x & 0xffffu); p = (int)it.y; pe = p + (int)(it.x >> 16); }
-                    const double acc = (own || eager) ? lu_diag_component(g, s, k, sub, p, pe) : 0.0;
-                    double a, b, c, d, y0, y1;
-                    cx.gather8(acc, a, b, c, d, y0, y1);
-                    if (own) lu_diag_finish(s, k, sub, a, b, c, d, y0, y1);
-                    else if (eager) *lu_component_cell(s, k, sub) = acc;
-                }
-            } else {
-                for (int idx = cx.tid; idx < n_items; idx += T) {
-                    if (idx < n_own) lu_diag_item(g, s, lb + idx);
-                    else lu_eager_item(g, s, g.eg_item[eb + idx - n_own]);
-                }
+            for (int idx = cx.tid; idx < n_items; idx += T) {
+                if (idx < n_own) lu_diag_item(g, s, lb + idx);
+                else lu_eager_item(g, s, g.eg_item[eb + idx - n_own]);
             }
             OPFG_TICK(112 + l);  // lane 0's own diagonal work (the rest of the phase: gathers of other lanes + barrier)
             // gathers of this level's off-diagonal items, from the far end of the lanes (the diagonals took the near end)
@@ -899,8 +805,8 @@ OPFG_HD void env_pf_solve(const GridDev& g, const C& cx, double* smem, const dou
 // scales, all from V and Ybus on the spot (the loads of V_k / V_child serve mismatch and Jacobian
 // alike).  Per environment only V, 1/|V|, t and W(k, parent) live in shared memory: 8.7 KB on the
 // 122-bus grid instead of 19 KB, and one phase per level instead of three plus a row pass.  The
-// smaller footprint is spent on MORE, NARROWER environments per SM: T = 8 / 16 / 32 lanes per
-// environment, several environments per warp, synchronised by __syncwarp alone (no block barriers).
+// smaller footprint is spent on MORE, NARROWER environments per SM: T = 16 lanes per
+// environment, two environments per warp, synchronised by __syncwarp alone (no block barriers).
 // Every sum runs in the order of env_pf_solve: same bits.
 struct TreeSmem { double *vri, *ivm, *t, *w0, *w1; };
 OPFG_HHD size_t tree_smem_doubles(int n, int nb) {
@@ -1039,36 +945,6 @@ OPFG_HD void env_pf_tree(const GridDev& g, const C& cx, double* smem, const doub
     // samples before).  Buses beyond OWN rounds (large grids) keep using the output buffers.
     constexpr int OWN = C::OWN_ROUNDS;       // 128 / T on the device: grids up to 128 buses stay in registers
     double vm_own[OWN], va_own[OWN];
-    const bool dc_here = g.init_dc && g.tr_dc;
-    if (dc_here) {
-        // pandapower init='dc' on a tree: B' theta = P needs no fill, so it is 2 x levels phases of a few scalar
-        // operations here instead of a dense GEMM launch of its own (k_dc_start) plus a round trip of the
-        // angles through HBM; the angles are left in s.t[2k]
-        for (int k = cx.tid; k < n; k += T) s.t[2 * k] = sbus[2 * g.tr_bus_of_int[k]] + g.tr_dc_rhs0[k];
-        cx.sync();
-        for (int l = 0; l < g.n_levels; ++l) {
-            const int le = g.tr_level_ptr[l + 1];
-            for (int k = g.tr_level_ptr[l] + cx.tid; k < le; k += T) {
-                double y = s.t[2 * k];
-                for (int e = g.tr_y_ptr[k] + 1; e < g.tr_y_ptr[k + 1]; ++e) {
-                    const uint32_t ent = g.tr_y_ent[e];
-                    if ((ent >> 16) == 1u) { const int j = (int)(ent & 0xffffu); y = fma(-g.tr_dc_w[j], s.t[2 * j], y); }
-                }
-                s.t[2 * k] = y;
-            }
-            cx.sync();
-        }
-        for (int l = g.n_levels - 1; l >= 0; --l) {
-            const int le = g.tr_level_ptr[l + 1];
-            for (int k = g.tr_level_ptr[l] + cx.tid; k < le; k += T) {
-                const int p = g.tr_parent[k];
-                double x = s.t[2 * k] * g.tr_dc_inv[k];
-                if (p >= 0) x = fma(-g.tr_dc_w[k], s.t[2 * p], x);
-                s.t[2 * k] = x;
-            }
-            cx.sync();
-        }
-    }
 #pragma unroll
     for (int r = 0; r < OWN; ++r) {
         const int i = cx.tid + r * T;
@@ -1077,7 +953,7 @@ OPFG_HD void env_pf_tree(const GridDev& g, const C& cx, double* smem, const doub
             const int bus = g.tr_bus_of_int[i];
             const double vm = g.vm_from_state ? vm_out[bus] : g.tr_vm0[i];
             const bool dead = ISL_T && g.isl && vm == 0.0;      // kernel 1 found the bus cut off from every slack
-            const double va = dead ? 0.0 : ((g.init_dc && i < n) ? (dc_here ? s.t[2 * i] : va_out[bus]) : g.tr_va0[i]);   // DC start: above, or the dense pre-pass wrote it
+            const double va = dead ? 0.0 : ((g.init_dc && i < n) ? va_out[bus] : g.tr_va0[i]);   // DC start: written by the dense pre-pass
             double sn, cs;
             sincos(va, &sn, &cs);
             vm_own[r] = vm; va_own[r] = va;
@@ -1089,7 +965,7 @@ OPFG_HD void env_pf_tree(const GridDev& g, const C& cx, double* smem, const doub
         const int bus = g.tr_bus_of_int[i];
         const double vm = g.vm_from_state ? vm_out[bus] : g.tr_vm0[i];
         const bool dead = ISL_T && g.isl && vm == 0.0;
-        const double va = dead ? 0.0 : ((g.init_dc && i < n) ? (dc_here ? s.t[2 * i] : va_out[bus]) : g.tr_va0[i]);
+        const double va = dead ? 0.0 : ((g.init_dc && i < n) ? va_out[bus] : g.tr_va0[i]);
         double sn, cs;
         sincos(va, &sn, &cs);
         if (live) { vm_out[bus] = vm; va_out[bus] = va; }
@@ -1502,14 +1378,14 @@ OPFG_HD void env_score(const GridDev& g, const C& cx, double* smem, const OpfgBa
     // the row is read piecemeal through references below: pull what will be read towards the SM now --
     // the observation runs if the observation is made of runs (the whole 10 KB row used to be fetched:
     // 348 MB per launch of 32 768 environments, two thirds of it never read), else the whole row
-    if (g.score_prefetch == 2 && g.n_obs_runs > 0) {
+    if (g.n_obs_runs > 0) {
         for (int r = 0; r < g.n_obs_runs; ++r) {
             const char* p0 = reinterpret_cast<const char*>(S + g.obs_runs[3 * r]);
             const int bytes = g.obs_runs[3 * r + 2] * 8;
             for (int off = cx.tid * 128; off < bytes + 127; off += T * 128)
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(p0 + (off < bytes ? off : bytes - 1)));
         }
-    } else if (g.score_prefetch != 0) {
+    } else {
         for (int off = cx.tid * 128; off < g.n_state * 8; off += T * 128)
             asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(S) + off));
     }

@@ -231,14 +231,10 @@ class BatchedOpfEnv:
         # first eligible reset is recorded, later ones replay the recording.  Only calls that go
         # through `_sample_keys` / `run_row_program` can be recorded, so hooks of user subclasses
         # (which may touch the state with arbitrary tensor code) have to opt in explicitly.
-        if fused_reset is None and os.environ.get("OPFG_FUSED_RESET"):
-            fused_reset = os.environ["OPFG_FUSED_RESET"] != "0"
         # Measured on B200 (VoltageControl): one launch beats six up to ~1.5k environments (+40 % at
         # 64-512), the separate full-occupancy kernels win beyond that -- hence the automatic rule.
         self.fused_reset = (type(self).__module__.startswith("opfgym_b200.") and self.num_envs <= 1024) \
             if fused_reset is None else bool(fused_reset)
-        if fuse_reset_obs is None and os.environ.get("OPFG_FUSE_RESET_OBS"):
-            fuse_reset_obs = os.environ["OPFG_FUSE_RESET_OBS"] != "0"
         self._fuse_reset_obs = type(self).__module__.startswith("opfgym_b200.") if fuse_reset_obs is None \
             else bool(fuse_reset_obs)
         self._reset_plans = {}
@@ -249,7 +245,6 @@ class BatchedOpfEnv:
             self._side = self.xp.cuda.Stream(device=self.device)
             self._copy_stream = self.xp.cuda.Stream(device=self.device)      # step_host: observation transfers
             self._pf_done = self.xp.cuda.Event()
-            self._late_prefetch = os.environ.get("OPFG_LATE_PREFETCH", "1") != "0"
             self._sampled_events = [self.xp.cuda.Event() for _ in range(3)]
             self._main_done = self.xp.cuda.Event()
             self._side_done = self.xp.cuda.Event()
@@ -857,21 +852,17 @@ class BatchedOpfEnv:
                 nxt = (e.cur + 1) % 3
                 pipe = dict(buf=nxt, obs="obs", ready=sample_ahead(nxt, h["obs"])())
             e.actions.copy_(src, non_blocking=True)    # this step's own work goes to the GPU first
-            if self._late_prefetch:
-                # The look-ahead episode is not needed before the NEXT call: its kernels are issued behind the
-                # power flow (the persistent kernel fills every SM, nothing runs beside it), where they share
-                # the GPU with kernel 5 and fill the gap between two calls -- 1.33 instead of 1.46 ms per call
-                # against issuing them at the start of the step, where they contend with kernel 1 / the DC GEMM
-                e.assemble()
-                e.pf_solve()
-                self._pf_done.record(main)
-                e.score(e.batch_final)
-            else:
-                e.step(final_obs=True)
+            # The look-ahead episode is not needed before the NEXT call: its kernels are issued behind the
+            # power flow (the persistent kernel fills every SM, nothing runs beside it), where they share
+            # the GPU with kernel 5 and fill the gap between two calls -- 1.33 instead of 1.46 ms per call
+            # against issuing them at the start of the step, where they contend with kernel 1 / the DC GEMM
+            e.assemble()
+            e.pf_solve()
+            self._pf_done.record(main)
+            e.score(e.batch_final)
             free = 3 - e.cur - pipe["buf"]             # the buffer of the episode before this one
             other = "obs_alt" if pipe["obs"] == "obs" else "obs"
-            copy_ahead = sample_ahead(free, h[other], after=self._results_copied,
-                                      start_after=self._pf_done if self._late_prefetch else None)
+            copy_ahead = sample_ahead(free, h[other], after=self._results_copied, start_after=self._pf_done)
         else:
             e.actions.copy_(src, non_blocking=True)
             e.step(final_obs=True)

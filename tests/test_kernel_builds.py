@@ -7,7 +7,7 @@ fails the case instead of passing it vacuously) and compares it with a second im
 * ``k_pf_multi`` (every stage level, threads per environment and launch bound) and ``k_pf`` (one CTA per
   environment) against ``k_pf_lanes``, the row-wise implementation of the same factorisation: bit for bit.
   Both engines use ordering 1 and the same threads per environment, hence the same schedule.
-* ``k_pf_tree`` (8 / 16 / 32 lanes, both 16-lane register builds) against the same: flag and iteration count
+* ``k_pf_tree`` (both register builds of its 16 lanes per environment) against the same: flag and iteration count
   exact, |V| and angle within 1e-11 (the radial kernel forms sum(L W) before subtracting it from J_kk).
 * ``k_score<T>`` and ``k_score_warps`` against the default scoring build of the grid.
 
@@ -16,11 +16,7 @@ U(5, 14) on HV grids).  Batches of 1, 3, 149 and 2051 environments leave environ
 half-warps idle; environments outside the batch must stay untouched.  The lane kernel itself is checked against
 the CPU oracle on a sample of the converged regime.
 """
-import concurrent.futures
 import functools
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -33,7 +29,6 @@ from opfgym_b200.compiler import Compiler
 from opfgym_b200.ppc import PpcBuilder
 from tests import common
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BATCHES = (1, 3, 149, 2051)
 N = max(BATCHES)
 MV, HV = "1-MV-semiurb--1-sw", "1-HV-urban--0-sw"
@@ -68,7 +63,7 @@ def _case(key):
 
 def _engine(key, monkeypatch, knobs=(), **kw):
     from opfgym_b200.engine import Engine
-    names = ("OPFG_STAGE", "OPFG_ENVS_PER_CTA", "OPFG_TREE_LANES", "OPFG_TREE_ENVS", "OPFG_SCORE_THREADS")
+    names = ("OPFG_STAGE", "OPFG_ENVS_PER_CTA", "OPFG_TREE_ENVS", "OPFG_SCORE_THREADS")
     for k in names:
         monkeypatch.delenv(k, raising=False)
     for k, v in dict(knobs).items():
@@ -265,36 +260,46 @@ def test_cta_case_table_hostsim(monkeypatch):
 
 
 # ---------------------------------------------------------------------------------------- radial builds
-# (grid, knobs, lanes, register build): 384 = the 16-lane build capped at 24 environments, 512 = the plain one
+# (grid, knobs, lanes, register build): 384 = the 16-lane build capped at 24 environments, 512 = the plain one.
+# Without a knob the 122-bus grid fits 24 environments per CTA, the 97-bus grid 32 and the 111-bus grid with taps 26.
+# Two environments per CTA (one warp) leave a CTA's last warp half idle whenever its share of the batch is odd.
 TREE_CASES = [
-    (MV, {"OPFG_TREE_LANES": 8}, 8, None),
-    (MV, {"OPFG_TREE_LANES": 16, "OPFG_TREE_ENVS": 24}, 16, 384),
-    (MV, {"OPFG_TREE_LANES": 32}, 32, None),
+    (MV, {"OPFG_TREE_ENVS": 24}, 16, 384),
+    (MV, {"OPFG_TREE_ENVS": 2}, 16, 384),
     ("1-MV-rural--0-sw", {}, 16, 512),
-    ("1-MV-rural--0-sw", {"OPFG_TREE_LANES": 8}, 8, None),
-    ("taps", {"OPFG_TREE_LANES": 8}, 8, None),
-    ("taps", {"OPFG_TREE_LANES": 16, "OPFG_TREE_ENVS": 24}, 16, 384),
-    ("taps", {"OPFG_TREE_LANES": 32}, 32, None),
+    ("1-MV-rural--0-sw", {"OPFG_TREE_ENVS": 24}, 16, 384),
+    ("1-MV-rural--0-sw", {"OPFG_TREE_ENVS": 2}, 16, 384),
+    ("taps", {}, 16, 512),
+    ("taps", {"OPFG_TREE_ENVS": 24}, 16, 384),
+    ("taps", {"OPFG_TREE_ENVS": 12}, 16, 384),
+    ("taps", {"OPFG_TREE_ENVS": 2}, 16, 384),
 ]
 TREE_WORST = {}
 
 
+def _tree_id(c):
+    envs = c[1].get("OPFG_TREE_ENVS", 24)
+    return f"{c[0][:8]}-L{c[2]}-{c[3]}" + ("" if envs == 24 else f"-E{envs}")
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("case", TREE_CASES, ids=[f"{c[0][:8]}-L{c[2]}-{c[3]}" for c in TREE_CASES])
+@pytest.mark.parametrize("case", TREE_CASES, ids=[_tree_id(c) for c in TREE_CASES])
 def test_radial_kernel_builds_match_lane_kernel(cuda_lib, monkeypatch, case):
     key, knobs, lanes, build = case
     eng = _engine(key, monkeypatch, knobs, ordering=1)
     info = eng.info
     assert info["pf_kernel_used"] == 3 and info["radial_lanes_per_env"] == lanes, info
     E = info["radial_envs_per_cta"]
-    assert E % (32 // lanes) == 0 and E <= (24 if lanes == 32 else 32), info
+    assert E % (32 // lanes) == 0 and E <= 32, info
+    if "OPFG_TREE_ENVS" in knobs:
+        assert E == knobs["OPFG_TREE_ENVS"], info
     if build == 384:
         assert E <= 24, info
     elif build == 512:
         assert E > 24, info
     if key == "taps":
         assert eng.yval is not None
-    TREE_WORST[(key, lanes, build)] = _compare(key, eng, 0, exact=False)
+    TREE_WORST[(key, E, build)] = _compare(key, eng, 0, exact=False)
     eng.close()
 
 
@@ -388,49 +393,3 @@ def test_scoring_builds_agree(cuda_lib, monkeypatch, case):
                 scale = np.abs(b[ok]).max(initial=0.0)
                 assert np.abs(a[ok] - b[ok]).max(initial=0.0) <= 1e-12 * scale, (regime, n, k)
     eng.close()
-
-
-# ------------------------------------------------------------------------------- knobs read once per process
-# `static` in the library: each setting runs in a process of its own (tests/_build_variant_run.py).  Register
-# caps and launch shapes change no arithmetic: every output bit must agree with the default build.
-VARIANTS = [
-    {"OPFG_AUX_WARPS": 1, "OPFG_ASSEMBLE_CAP": 3, "OPFG_SCORE_CAP": 3},
-    {"OPFG_ASSEMBLE_CAP": 1, "OPFG_SCORE_CAP": 1},
-    {"OPFG_ASSEMBLE_CAP": 2, "OPFG_SCORE_CAP": 4},
-    {"OPFG_SCORE_CAP": 0, "OPFG_TREE_WIDE_REGS": 0, "OPFG_MULTI_ROOMY": 0},
-    {"OPFG_PREFER_ENVS": 0},
-]
-VARIANT_BASE = {"OPFG_TREE_ENVS": 24}        # the 122-bus grid then runs the 16-lane build TREE_WIDE_REGS selects
-
-
-@pytest.mark.gpu
-def test_process_wide_knobs_change_no_bit(cuda_lib, monkeypatch, tmp_path):
-    from tests import _build_variant_run as helper
-    for k, v in VARIANT_BASE.items():
-        monkeypatch.setenv(k, str(v))
-    base = helper.run_all()
-    info = {k: base.pop(k) for k in list(base) if k.endswith("/info")}
-
-    def child(i):
-        env = dict(os.environ)
-        env.update({k: str(v) for k, v in {**VARIANT_BASE, **VARIANTS[i]}.items()})
-        out = tmp_path / f"variant{i}.npz"
-        flags = ["-s"] if sys.flags.no_user_site else []
-        res = subprocess.run([sys.executable, *flags, os.path.join(ROOT, "tests", "_build_variant_run.py"), str(out)],
-                             env=env, cwd=ROOT, capture_output=True, text=True, timeout=600)
-        assert res.returncode == 0, (VARIANTS[i], res.stderr[-3000:])
-        return dict(np.load(out))
-
-    with concurrent.futures.ThreadPoolExecutor(len(VARIANTS)) as pool:
-        results = list(pool.map(child, range(len(VARIANTS))))
-    for knobs, got in zip(VARIANTS, results):
-        got_info = {k: got.pop(k) for k in list(got) if k.endswith("/info")}
-        assert set(got) == set(base)
-        for k in base:
-            assert np.array_equal(got[k].view(np.uint8), base[k].view(np.uint8)), (knobs, k)
-        if "OPFG_PREFER_ENVS" in knobs:     # the knob applies: the 372-bus grid stages every table for 2 environments
-            assert tuple(info[f"{HV}/info"][:3]) == (1, 3, 0), info
-            assert tuple(got_info[f"{HV}/info"][:3]) == (1, 2, 2), got_info
-        else:
-            for k in info:
-                assert np.array_equal(info[k], got_info[k]), (knobs, k)

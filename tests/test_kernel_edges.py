@@ -27,13 +27,10 @@ DC_GRIDS = ("1-MV-rural--0-sw", "1-MV-comm--2-sw", "1-MV-semiurb--1-sw", "1-HV-u
 DC_BATCHES = (1, 2, 127, 128, 129, 1000, 4133)
 DC_BATCHES_HOST = (1, 2, 129)
 N_INPUT = max(DC_BATCHES)
-# name -> (pf_kernel, environment knobs, pf_kernel_used, launches per opfg_pf_solve)
-#   prepass      the GEMM pre-pass (default) in front of whatever kernel auto picks (radial kernel on radial grids)
+# name -> (pf_kernel, pf_kernel_used); every path launches the GEMM pre-pass, then the power-flow kernel
+#   prepass      the GEMM pre-pass in front of whatever kernel auto picks (radial kernel on radial grids)
 #   prepass_cta  the GEMM pre-pass in front of the CTA kernel
-#   in_cta       OPFG_DC_PREPASS=0: the sparse DC solve inside env_pf_solve
-#   in_tree      OPFG_TREE_DC=1: the leaf-first DC solve inside the radial kernel
-DC_PATHS = {"prepass": ("auto", {}, None, 2), "prepass_cta": ("cta", {}, 1, 2),
-            "in_cta": ("auto", {"OPFG_DC_PREPASS": "0"}, 1, 1), "in_tree": ("auto", {"OPFG_TREE_DC": "1"}, 3, 1)}
+DC_PATHS = {"prepass": ("auto", None), "prepass_cta": ("cta", 1)}
 
 
 @functools.lru_cache(maxsize=None)
@@ -69,18 +66,12 @@ def _radial(name):
 
 
 def _paths(name):
-    return [p for p in DC_PATHS if _radial(name) or p in ("prepass", "in_cta")]
+    return [p for p in DC_PATHS if _radial(name) or p == "prepass"]
 
 
-def _dc_engine(engine_cls, name, path, monkeypatch, n=N_INPUT):
-    pf_kernel, knobs, used, _ = DC_PATHS[path]
-    for k in ("OPFG_DC_PREPASS", "OPFG_TREE_DC"):
-        monkeypatch.delenv(k, raising=False)
-    for k, v in knobs.items():
-        monkeypatch.setenv(k, v)           # read when the grid is created
+def _dc_engine(engine_cls, name, path, n=N_INPUT):
+    pf_kernel, used = DC_PATHS[path]
     eng = engine_cls(_case(name).program, n, max_iteration=0, pf_kernel=pf_kernel)
-    for k in knobs:
-        monkeypatch.delenv(k)
     expect = used if used is not None else (3 if _radial(name) else 1)
     assert eng.info["pf_kernel_used"] == expect, (name, path, eng.info)
     return eng
@@ -108,7 +99,7 @@ def _check_dc(eng, name, path, batches, sync=lambda: None):
     for n in batches:
         va, launches = _dc_run(eng, sbus, n, sync)
         if not isinstance(eng.va, np.ndarray):
-            assert launches == DC_PATHS[path][3], (path, launches)      # the pre-pass ran (or did not)
+            assert launches == 2, (path, launches)                     # the pre-pass ran
         assert np.isfinite(va).all()
         err = np.abs(va - want[:n]).max()
         assert err <= 1e-11, (name, path, n, err)
@@ -118,28 +109,27 @@ def _check_dc(eng, name, path, batches, sync=lambda: None):
 
 
 @pytest.mark.parametrize("name", DC_GRIDS)
-def test_dc_start_matches_scipy_hostsim(name, monkeypatch):
+def test_dc_prepass_matches_scipy_hostsim(name):
     for path in _paths(name):
-        eng = _dc_engine(harness.HostSimEngine, name, path, monkeypatch, n=max(DC_BATCHES_HOST))
+        eng = _dc_engine(harness.HostSimEngine, name, path, n=max(DC_BATCHES_HOST))
         _check_dc(eng, name, path, DC_BATCHES_HOST)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", DC_GRIDS)
-def test_dc_start_matches_scipy_and_host_loop_cuda(cuda_lib, name, monkeypatch):
+def test_dc_prepass_matches_scipy_and_host_loop_cuda(cuda_lib, name):
     """Every DC path within 1e-11 rad of scipy; the GEMM pre-pass equal, value for value, to the host build's
     plain loop (both accumulate fma(P, Binv, acc) in bus order; a padded term is fma(0, 0, acc))."""
     import torch
     from opfgym_b200.engine import Engine
     sbus = _dc_inputs(name)[0]
     for path in _paths(name):
-        eng = _dc_engine(Engine, name, path, monkeypatch)
+        eng = _dc_engine(Engine, name, path)
         got = _check_dc(eng, name, path, DC_BATCHES, sync=torch.cuda.synchronize)
-        if DC_PATHS[path][3] == 2:              # the GEMM pre-pass produced the start
-            # the same configuration on the host: B'^-1 is built with the factor of the grid's own ordering
-            want_host, _ = _dc_run(_dc_engine(harness.HostSimEngine, name, path, monkeypatch), sbus, N_INPUT)
-            for n, va in got.items():
-                assert (va == want_host[:n]).all(), (name, path, n)
+        # the same configuration on the host: B'^-1 is built with the factor of the grid's own ordering
+        want_host, _ = _dc_run(_dc_engine(harness.HostSimEngine, name, path), sbus, N_INPUT)
+        for n, va in got.items():
+            assert (va == want_host[:n]).all(), (name, path, n)
         eng.close()
 
 

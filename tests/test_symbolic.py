@@ -106,26 +106,21 @@ def test_bad_tables_are_rejected():
 
 @pytest.mark.parametrize("name", ["1-MV-semiurb--1-sw", "1-HV-urban--0-sw"])
 def test_dense_dc_prepass_equals_sparse_dc_start(name, monkeypatch):
-    """The DC start as a dense pre-pass (B'^-1 built on the host with the kernel's factor) and as the
-    level-scheduled sparse solve inside the kernel seed the same Newton iteration; so do the schedule
-    with and without the eager gather of far Schur updates (bit-identical by construction)."""
+    """The schedule with and without the eager gather of far Schur updates seeds and runs the same Newton
+    iteration, bit for bit (the partial sums keep the order of additions of the single gather).  The DC start
+    comes from the dense pre-pass in both runs; the CTA kernel is the one that runs the schedule."""
     from tests import common
     from tests.hostsim.harness import HostSimEngine
     case = common.make_case(name)
     results = {}
-    for label, env in (("dense", {"OPFG_DC_PREPASS": "1", "OPFG_EAGER_GATHER": "0"}),
-                       ("sparse", {"OPFG_DC_PREPASS": "0", "OPFG_EAGER_GATHER": "0"}),
-                       ("sparse+eager", {"OPFG_DC_PREPASS": "0", "OPFG_EAGER_GATHER": "1"})):
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        eng = HostSimEngine(case.program, 6)
+    for eager in ("0", "1"):
+        monkeypatch.setenv("OPFG_EAGER_GATHER", eager)
+        eng = HostSimEngine(case.program, 6, pf_kernel="cta")
+        assert eng.info["pf_kernel_used"] == 1, eng.info
         common.randomize(case, eng, seed=5)
         eng.assemble()
         eng.pf_solve()
-        results[label] = (eng.converged.copy(), eng.iterations.copy(), eng.vm.copy(), eng.va.copy())
-    dense, sparse, eager = results["dense"], results["sparse"], results["sparse+eager"]
-    assert dense[0].all() and (dense[0] == sparse[0]).all() and (dense[1] == sparse[1]).all()
-    np.testing.assert_allclose(dense[2], sparse[2], rtol=0, atol=1e-11)
-    np.testing.assert_allclose(dense[3], sparse[3], rtol=0, atol=1e-11)
-    for a, b in zip(sparse, eager):
+        results[eager] = (eng.converged.copy(), eng.iterations.copy(), eng.vm.copy(), eng.va.copy())
+    assert results["0"][0].all()
+    for a, b in zip(results["0"], results["1"]):
         assert np.array_equal(a, b)
