@@ -1138,12 +1138,23 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
             std::vector<double> qmn, qmx;
             if (desc->enforce_q_lims && desc->gen_cols > OPFG_QMIN) {
                 std::vector<double> mn(nb, 0.0), mx(nb, 0.0);
-                std::vector<int> cnt(nb, 0);
+                std::vector<int> cnt(nb, 0), first(nb, -1);
                 for (int gI = 0; gI < ng; ++gI) {
                     const double* row = desc->gen + (size_t)gI * desc->gen_cols;
                     const int bus = (int)row[OPFG_GEN_BUS];
                     if (row[OPFG_GEN_STATUS] <= 0 || type[bus] != 2) continue;
-                    if (row[OPFG_QMAX] == 0.0 && row[OPFG_QMIN] == 0.0) continue;   // pandapower's both-zero rule
+                    // the limits of a bus are pooled into one sum, which equals pandapower's per-generator check
+                    // (equal shares of the bus Q) only when every generator of the bus has the same pair
+                    if (first[bus] < 0) first[bus] = gI;
+                    const double* r0 = desc->gen + (size_t)first[bus] * desc->gen_cols;
+                    if (first[bus] != gI && (r0[OPFG_QMIN] != row[OPFG_QMIN] || r0[OPFG_QMAX] != row[OPFG_QMAX])) {
+                        delete G;
+                        return fail("enforce_q_lims: generator rows %d and %d of PV bus %d (ppc numbering) have different reactive "
+                                    "limits (%g, %g) and (%g, %g) MVAr; per-generator limits on one bus are not supported",
+                                    first[bus], gI, bus, r0[OPFG_QMIN], r0[OPFG_QMAX], row[OPFG_QMIN], row[OPFG_QMAX]);
+                    }
+                    // pandapower skips a generator with a zero limit (non_refs = (QMAX != 0) & (QMIN != 0))
+                    if (row[OPFG_QMAX] == 0.0 || row[OPFG_QMIN] == 0.0) continue;
                     mn[bus] += row[OPFG_QMIN] / base; mx[bus] += row[OPFG_QMAX] / base; cnt[bus]++;
                 }
                 for (int b = 0; b < nb; ++b)

@@ -65,8 +65,8 @@ struct GridDev {
     const double* bus_ysh;             // [nb*2] (GS + jBS)/base by ppc bus
     const int* br_f;                   // [nbr] ppc from bus
     const int* br_t;
-    // enforce_q_lims: PV buses whose generators have active reactive limits (both-zero limits are
-    // skipped like pandapower does); limits are per bus, in p.u. of base_mva
+    // enforce_q_lims: PV buses whose generators have active reactive limits (a generator with a zero
+    // limit is skipped like pandapower does); limits are per bus, in p.u. of base_mva
     int n_qlim;
     const int* qlim_bus;               // [n_qlim] internal bus index
     const double *qlim_min, *qlim_max; // [n_qlim]

@@ -36,7 +36,9 @@ oracle/pf.py (none could be checked here: pandapower is not installed):
     vm_pu set-points, gen/ext-grid buses at their set-point.
  6. max_iteration='auto' -> 10, tolerance_mva=1e-8 compared against the
     per-unit mismatch (identical for sn_mva=1, the SimBench value).
- 7. enforce_q_lims skips generators whose QMIN and QMAX are both 0.
+ 7. enforce_q_lims skips generators with QMIN == 0 or QMAX == 0 (pandapower's
+    `non_refs = (QMAX != 0) & (QMIN != 0)`).  The in-service generators of one PV
+    bus must share one (QMIN, QMAX) pair; other pairs are rejected by the engine.
  8. trafo_loading='current'.
  9. trafo3w (build_branch._trafo_df_from_trafo3w): one auxiliary star-point bus and three 2-winding
     equivalent branches hv->star, star->mv, star->lv, stacked behind the trafos in three blocks (all hv

@@ -204,7 +204,7 @@ def run_pf(ppc: Ppc, tolerance_mva=1e-8, max_iteration=10, enforce_q_lims=True,
             gen[at[0], PG] = sinj.real[r] - gen[at[1:], PG].sum()
         if not (ok and enforce_q_lims):
             break
-        # pandapower _run_ac_pf_with_qlims_enforced: both-zero limits are skipped
+        # pandapower _run_ac_pf_with_qlims_enforced: a generator with QMAX == 0 or QMIN == 0 is skipped
         lim = (gen[:, QMAX] != 0.0) & (gen[:, QMIN] != 0.0) & on & (bus[gbus, BUS_TYPE] == PV)
         mx = np.nonzero(lim & (gen[:, QG] > gen[:, QMAX]))[0]
         mn = np.nonzero(lim & (gen[:, QG] < gen[:, QMIN]))[0]

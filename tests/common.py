@@ -28,7 +28,7 @@ class Case:
 
 
 def make_case(name="1-MV-semiurb--1-sw", n_profile_steps=672, reward=None, constraint_kwargs=None,
-              load_scaling=1.5, gen_scaling=1.3, tight=False, prepare=None) -> Case:
+              load_scaling=1.5, gen_scaling=1.3, tight=False, prepare=None, extra_obs=()) -> Case:
     net, _ = grids.build_simbench_net(name, n_profile_steps=n_profile_steps,
                                       load_scaling=load_scaling, gen_scaling=gen_scaling)
     if prepare is not None:      # net tweaks before the tables are compiled (e.g. generator Q limits)
@@ -55,7 +55,8 @@ def make_case(name="1-MV-semiurb--1-sw", n_profile_steps=672, reward=None, const
                 ("load", "p_mw", net.load.index), ("load", "q_mvar", net.load.index),
                 ("res_bus", "vm_pu", net.bus.index[:5]),
                 ("res_line", "loading_percent", net.line.index[:4]),
-                ("res_ext_grid", "p_mw", net.ext_grid.index)]
+                ("res_ext_grid", "p_mw", net.ext_grid.index)] + \
+        [(t, c, net[t[len("res_"):]].index) for t, c in extra_obs]      # result columns of every element
     act_keys = [("sgen", "q_mvar", ctrl)]
     cons = CN.create_default_constraints(net, constraint_kwargs or {})
     rf = reward or RW.Summation()
@@ -112,7 +113,7 @@ def oracle_env(case: Case, eng, b: int):
     out = {"net": net}
     try:
         res = pf.runpp(net)            # the oracle's own net -> ppc conversion (oracle/ppc_ref.py)
-        out.update(converged=True, iterations=res["iterations"],
+        out.update(converged=True, iterations=res["iterations"], pf=res,
                    vm=net.res_bus.vm_pu.to_numpy(float), va=np.radians(net.res_bus.va_degree.to_numpy(float)))
         out.update(scoring.step_reward(net, case.constraints, case.reward))
         obs = [net[t].loc[idxs, c].to_numpy(float) for t, c, idxs in case.obs_keys]

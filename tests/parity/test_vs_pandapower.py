@@ -30,6 +30,12 @@ def _nets():
     same_level = [b for b in extra.bus.index if extra.bus.vn_kv[b] == extra.bus.vn_kv[10] and b != 10]
     pp.create_impedance(extra, 10, same_level[-1], rft_pu=0.02, xft_pu=0.07, sn_mva=50.0)
     yield "case14+ward+impedance", extra
+    # one-sided generator Q limits (pandapower skips a generator with QMIN == 0 or QMAX == 0) next to tight two-sided
+    # ones that bind: pins the skip rule of oracle/pf.py and of the engine's q-limit tables
+    one_sided = pn.case14()
+    one_sided.gen["min_q_mvar"] = [0.0, -5.0, -3.0, -3.0][:len(one_sided.gen)]
+    one_sided.gen["max_q_mvar"] = [5.0, 0.0, 3.0, 3.0][:len(one_sided.gen)]
+    yield "case14+one-sided-q-limits", one_sided
     try:
         import simbench as sb
         yield "1-MV-semiurb--1-sw", sb.get_simbench_net("1-MV-semiurb--1-sw")

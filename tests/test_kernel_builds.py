@@ -15,6 +15,11 @@ Two input regimes: converged, and across the collapse boundary (injections scale
 U(5, 14) on HV grids).  Batches of 1, 3, 149 and 2051 environments leave environment groups, CTA shares and radial
 half-warps idle; environments outside the batch must stay untouched.  The lane kernel itself is checked against
 the CPU oracle on a sample of the converged regime.
+
+Three grids carry generator Q limits that bind in part of the batch (enforce_q_lims, the QLIM builds): the 372-bus
+grid, the 355-bus grid (odd bus count) and the 372-bus grid with tap actions (per-environment Ybus values).  There
+the matrix also asserts that the PV->PQ restart really runs, and the lane kernel's switched buses, |V|, angle and
+generator Q are held against the oracle's q-limit loop.
 """
 import functools
 
@@ -23,25 +28,51 @@ import pytest
 
 from opfgym_b200 import capi
 from opfgym_b200 import grids
+from opfgym_b200 import net as pn
 from opfgym_b200 import constraints as CN
 from opfgym_b200 import reward as RW
 from opfgym_b200.compiler import Compiler
-from opfgym_b200.ppc import PpcBuilder
+from opfgym_b200.ppc import BUS_TYPE, PQ, PV, VM, PpcBuilder
 from tests import common
 
 BATCHES = (1, 3, 149, 2051)
 N = max(BATCHES)
 MV, HV = "1-MV-semiurb--1-sw", "1-HV-urban--0-sw"
-LAM = {MV: (5.0, 12.0), HV: (5.0, 14.0), "taps": (5.0, 12.0), "1-MV-rural--0-sw": (2.0, 6.0)}
+LAM = {MV: (5.0, 12.0), HV: (5.0, 14.0), "taps": (5.0, 12.0), "1-MV-rural--0-sw": (2.0, 6.0),
+       "hvq": (5.0, 14.0), "hvq355": (2.0, 6.0), "hvq-taps": (5.0, 14.0)}
 PF_TOL = dict(vm=1e-6, va=1e-6, loading=1e-4, reward_rel=1e-6)        # tests/test_gpu_parity.py
 
 
-def _taps_case():
-    """The 111-bus grid with transformer tap actions: the Ybus values are per environment (MODE 4-6 of k_pf_multi,
-    the DYN builds of k_pf, k_pf_tree and k_pf_lanes).  With tap cells only the grid stays radial and no outage can
-    island a bus, so the lane kernel runs there as the reference.  (Switchable ties would make every line's
-    in_service a cell and turn the island walk on, and the lane kernel has no island handling.)"""
-    net, _ = grids.build_simbench_net("1-MV-comm--2-sw", n_profile_steps=96, load_scaling=1.5, gen_scaling=1.3)
+def _q_limits(lims):
+    """Heterogeneous generator Q limits [MVAr], each binding in part of the batch; NaN (no limit) becomes +-1e9."""
+    def prepare(net):
+        if len(net.gen) == 0:      # the 355-bus grid has none: five at fixed 110-kV buses
+            for b, p in ((40, 30.0), (95, 45.0), (160, 25.0), (230, 50.0), (310, 35.0)):
+                pn.create_gen(net, b, p_mw=p, vm_pu=1.0)
+        net.gen["min_q_mvar"] = [lo for lo, _ in lims]
+        net.gen["max_q_mvar"] = [hi for _, hi in lims]
+        net.gen["vm_pu"] = np.linspace(0.99, 1.03, len(net.gen))
+    return prepare
+
+
+HVQ_LIMITS = [(np.nan, np.nan), (-65.0, 25.0), (-8.0, 81.0), (-30.0, 30.0), (-20.0, 105.0)]
+HVQ355_LIMITS = [(-150.0, 50.0), (-15.0, 50.0), (np.nan, np.nan), (-30.0, 30.0), (-5.0, 160.0)]
+
+
+# grids with generator Q limits that bind (enforce_q_lims: the QLIM builds of every power-flow kernel but the radial one)
+QLIM_GRIDS = {"hvq": (HV, _q_limits(HVQ_LIMITS)), "hvq355": ("1-HV-mixed--1-sw", _q_limits(HVQ355_LIMITS))}
+QLIM_KEYS = tuple(QLIM_GRIDS) + ("hvq-taps",)
+
+
+def _taps_case(name="1-MV-comm--2-sw", prepare=None):
+    """A grid with transformer tap actions: the Ybus values are per environment (MODE 4-6 of k_pf_multi, the DYN
+    builds of k_pf, k_pf_tree and k_pf_lanes).  With tap cells only no outage can island a bus, so the lane kernel
+    runs there as the reference.  (Switchable ties would make every line's in_service a cell and turn the island
+    walk on, and the lane kernel has no island handling.)  The 111-bus grid stays radial; the 372-bus grid's tap
+    changers sit on the HV side of its 380/110-kV transformers."""
+    net, _ = grids.build_simbench_net(name, n_profile_steps=96, load_scaling=1.5, gen_scaling=1.3)
+    if prepare is not None:
+        prepare(net)
     net.trafo["min_tap_pos"] = -3.0
     net.trafo["max_tap_pos"] = 3.0
     act_keys = [("trafo", "tap_pos", net.trafo.index)]
@@ -58,6 +89,11 @@ def _taps_case():
 def _case(key):
     if key == "taps":
         return _taps_case()
+    if key == "hvq-taps":
+        return _taps_case(HV, prepare=_q_limits(HVQ_LIMITS))
+    if key in QLIM_GRIDS:
+        return common.make_case(QLIM_GRIDS[key][0], n_profile_steps=96, prepare=QLIM_GRIDS[key][1],
+                                extra_obs=[("res_gen", "q_mvar")])
     return common.make_case(key, n_profile_steps=96)
 
 
@@ -100,7 +136,7 @@ def _inputs(key):
     if eng.yval is not None:
         for r in out.values():
             r["yval"] = eng.yval.clone()
-    if key != "taps":      # (tests/test_dynamic_branches.py replays tap actions on the oracle)
+    if key not in ("taps", "hvq-taps"):      # (tests/test_dynamic_branches.py replays tap actions on the oracle)
         eng.pf_solve()
         eng.score()
         _sync()
@@ -109,8 +145,53 @@ def _inputs(key):
         assert worst["flag_mismatch"] == worst["iter_mismatch"] == worst["valid_mismatch"] == 0, worst
         for k, tol in PF_TOL.items():
             assert worst[k] <= tol, (k, worst)
+        if key in QLIM_GRIDS:
+            _check_q_limits_with_oracle(case, eng, range(5, N, 128))
     eng.close()
     return out
+
+
+def _switched(ppc, vm):
+    """PV buses and [envs, PV buses] True where a PV bus's |V| left its set-point.  Both solvers add exactly 0.0 to
+    the |V| of a PV bus in every update, so a bus that never switched to PQ keeps its set-point bit for bit."""
+    pv = np.nonzero(ppc.bus[:, BUS_TYPE] == PV)[0]
+    return pv, vm[:, pv] != ppc.bus[pv, VM]
+
+
+def _check_q_limits_with_oracle(case, eng, envs):
+    """Per environment against the oracle's q-limit loop: flag and iteration count exact, the same PV buses
+    switched to PQ, |V| and angle within 1e-9, generator Q within 1e-6 MVAr (a switched generator reports its
+    limit)."""
+    ppc = case.program.ppc
+    lk = ppc.bus_lookup
+    has = lk >= 0
+    vm, va = common._np(eng.vm), common._np(eng.va)
+    conv, iters = common._np(eng.converged), common._np(eng.iterations)
+    q_eng = common._np(eng.column("res_gen", "q_mvar"))
+    pv, sw = _switched(ppc, vm)
+    gen = case.net.gen
+    lo = np.where(np.isnan(gen.min_q_mvar), -1e9, gen.min_q_mvar)
+    hi = np.where(np.isnan(gen.max_q_mvar), 1e9, gen.max_q_mvar)
+    gen_pos = case.net.bus.index.get_indexer(gen.bus)
+    n_switched = 0
+    for b in envs:
+        o = common.oracle_env(case, eng, b)
+        assert o["converged"] and bool(conv[b]) and iters[b] == o["iterations"], (b, iters[b], o.get("iterations"))
+        res = o["pf"]
+        olk = res["ppc"].bus_lookup
+        o_sw = (res["ppc"].bus[:, BUS_TYPE] == PV) & (res["bus"][:, BUS_TYPE] == PQ)
+        e_sw = np.zeros(ppc.bus.shape[0], bool)
+        e_sw[pv] = sw[b]
+        assert np.array_equal(e_sw[lk[has]], o_sw[olk[has]]), b
+        n_switched += int(e_sw.sum())
+        assert np.abs(vm[b][lk[has]] - o["vm"][has]).max() <= 1e-9, b
+        assert np.abs(va[b][lk[has]] - o["va"][has]).max() <= 1e-9, b
+        q_ref = o["net"].res_gen.q_mvar.to_numpy()
+        assert np.abs(q_eng[b] - q_ref).max() <= 1e-6, (b, q_eng[b], q_ref)
+        at = e_sw[lk[gen_pos]]
+        at_limit = np.minimum(np.abs(q_eng[b] - lo), np.abs(q_eng[b] - hi)) <= 1e-6
+        assert at_limit[at].all(), (b, q_eng[b])
+    assert n_switched > 0
 
 
 def _solve(eng, inp, n):
@@ -146,6 +227,11 @@ def _reference(key, threads):
     eng.close()
     assert ref["converged"]["converged"].all()
     assert 0.1 < ref["collapse"]["converged"].mean() < 0.9
+    if key in QLIM_KEYS:       # the q-limit restart really runs: some environments switch buses, others none
+        ok = ref["converged"]["converged"].astype(bool)
+        n_sw = _switched(_case(key).program.ppc, ref["converged"]["vm"])[1][ok].sum(axis=1)
+        assert 0.1 < (n_sw >= 1).mean() < 0.9, np.bincount(n_sw)
+        assert (n_sw >= 2).any(), np.bincount(n_sw)
     return ref
 
 
@@ -210,12 +296,47 @@ CTA_CASES = [
     ("taps", 0, {"OPFG_STAGE": 1, "OPFG_ENVS_PER_CTA": 4}, 64, 4, 1),
     ("taps", 0, {"OPFG_ENVS_PER_CTA": 1}, 64, 1, None),
     ("taps", 128, {"OPFG_ENVS_PER_CTA": 1}, 128, 1, None),
+    # generator Q limits that bind: the restart of the q-limit outer loop, its tables staged at stage 2; every
+    # (stage, launch bound) the shared-memory budget reaches (two environments at most once the tables are staged)
+    ("hvq", 0, {}, 128, 3, 0),
+    ("hvq", 0, {"OPFG_STAGE": 1}, 128, 2, 1),
+    ("hvq", 0, {"OPFG_STAGE": 2}, 128, 2, 2),
+    ("hvq", 32, {}, 32, 3, 0),
+    ("hvq", 64, {"OPFG_STAGE": 2}, 64, 2, 2),
+    ("hvq", 64, {"OPFG_ENVS_PER_CTA": 2, "OPFG_STAGE": 0}, 64, 2, 0),
+    ("hvq", 256, {}, 256, 3, 0),
+    ("hvq", 256, {"OPFG_STAGE": 1}, 256, 2, 1),
+    ("hvq", 256, {"OPFG_STAGE": 2}, 256, 2, 2),
+    ("hvq", 0, {"OPFG_ENVS_PER_CTA": 1}, 128, 1, None),
+    ("hvq", 64, {"OPFG_ENVS_PER_CTA": 1}, 64, 1, None),
+    # odd bus count: env_pf_solve's q-limit scratch starts one double past the reduction scratch
+    ("hvq355", 0, {}, 128, 3, 0),
+    ("hvq355", 0, {"OPFG_STAGE": 1}, 128, 2, 1),
+    ("hvq355", 0, {"OPFG_STAGE": 2}, 128, 2, 2),
+    ("hvq355", 32, {"OPFG_STAGE": 2}, 32, 2, 2),
+    ("hvq355", 64, {}, 64, 3, 0),
+    ("hvq355", 256, {"OPFG_STAGE": 1}, 256, 2, 1),
+    ("hvq355", 256, {"OPFG_STAGE": 2}, 256, 2, 2),
+    ("hvq355", 0, {"OPFG_ENVS_PER_CTA": 1}, 128, 1, None),
+    ("hvq355", 32, {"OPFG_ENVS_PER_CTA": 1}, 32, 1, None),
+    # per-environment Ybus values together with the q-limit loop (MODE 4-6, lane MODE 6/7)
+    ("hvq-taps", 0, {}, 128, 3, 0),
+    ("hvq-taps", 0, {"OPFG_STAGE": 1}, 128, 2, 1),
+    ("hvq-taps", 0, {"OPFG_STAGE": 2}, 128, 2, 2),
+    ("hvq-taps", 32, {}, 32, 3, 0),
+    ("hvq-taps", 64, {"OPFG_STAGE": 1}, 64, 2, 1),
+    ("hvq-taps", 256, {}, 256, 3, 0),
+    ("hvq-taps", 256, {"OPFG_STAGE": 1}, 256, 2, 1),
+    ("hvq-taps", 256, {"OPFG_STAGE": 2}, 256, 2, 2),
+    ("hvq-taps", 0, {"OPFG_ENVS_PER_CTA": 1}, 128, 1, None),
+    ("hvq-taps", 64, {"OPFG_ENVS_PER_CTA": 1}, 64, 1, None),
 ]
 
 
 def _cta_id(c):
     key, threads, knobs, _, E, stage = c
-    name = {MV: "mv122", HV: "hv372", "taps": "taps111"}[key]
+    name = {MV: "mv122", HV: "hv372", "taps": "taps111", "hvq": "hvq372", "hvq355": "hvq355",
+            "hvq-taps": "hvqtaps372"}[key]
     return f"{name}-T{threads or 'auto'}-E{E}-S{stage}"
 
 
@@ -236,12 +357,22 @@ def test_cta_kernel_builds_match_lane_kernel(cuda_lib, monkeypatch, case):
 
 def test_cta_cases_cover_every_stage_and_launch_bound():
     """The table above reaches every (stage, launch bound) instantiation of k_pf_multi, every stage with
-    per-environment Ybus, and k_pf for T = 64 and 128 with and without per-environment Ybus."""
-    seen = {(key == "taps", "k_pf" if E == 1 else stage, T if E == 1 else _bound(T, E))
-            for key, _, _, T, E, stage in CTA_CASES}
+    per-environment Ybus, and k_pf for T = 64 and 128 with and without per-environment Ybus.  With generator Q
+    limits that bind: every stage with and without per-environment Ybus, every launch bound the budget reaches
+    (stage 0 at 256, 384 and 768; staged tables leave room for two environments: 256 and 768), every thread count
+    on both bus-count parities, and k_pf for two thread counts with and without per-environment Ybus."""
+    seen = {(key in ("taps", "hvq-taps"), "k_pf" if E == 1 else stage, T if E == 1 else _bound(T, E))
+            for key, _, _, T, E, stage in CTA_CASES if key not in QLIM_KEYS}
     want = {(False, s, b) for s in (0, 1, 2) for b in (256, 384, 768)} | {(True, s, 768) for s in (0, 1, 2)} | \
         {(d, "k_pf", T) for d in (False, True) for T in (64, 128)}
     assert want <= seen, want - seen
+    seen_q = {(key == "hvq-taps", "k_pf" if E == 1 else stage, T if E == 1 else _bound(T, E))
+              for key, _, _, T, E, stage in CTA_CASES if key in QLIM_KEYS}
+    want_q = {(d, s, b) for d in (False, True) for s in (0, 1, 2) for b in (256, 768)} | \
+        {(d, 0, 384) for d in (False, True)} | {(d, "k_pf", T) for d in (False, True) for T in (64, 128)}
+    assert want_q <= seen_q, want_q - seen_q
+    for key in ("hvq", "hvq355"):
+        assert {T for k, _, _, T, _, _ in CTA_CASES if k == key} == {32, 64, 128, 256}, key
 
 
 def test_cta_case_table_hostsim(monkeypatch):
@@ -304,7 +435,9 @@ def test_radial_kernel_builds_match_lane_kernel(cuda_lib, monkeypatch, case):
 
 
 # ---------------------------------------------------------------------------------------- scoring builds
-SCORE_CASES = [(MV, None, 32), (MV, 64, 64), (MV, 128, 128), (MV, 256, 256), (HV, None, 128), (HV, 32, 32)]
+# hvq: kernel 5 on states where generators sit at their Q limits (res_gen.q_mvar is one of its observations)
+SCORE_CASES = [(MV, None, 32), (MV, 64, 64), (MV, 128, 128), (MV, 256, 256), (HV, None, 128), (HV, 32, 32),
+               ("hvq", None, 128), ("hvq", 32, 32)]
 SCORE_BATCHES = (1, 3, 2051)
 EXACT_STATS = [0, 1, 2, 7] + list(range(8, capi.N_STATS))     # counts: N, converged, valid, iterations, violated
 
@@ -367,12 +500,12 @@ def _score_reference(key):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("case", SCORE_CASES, ids=[f"{'mv122' if c[0] == MV else 'hv372'}-{c[1] or 'default'}"
+@pytest.mark.parametrize("case", SCORE_CASES, ids=[f"{ {MV: 'mv122', HV: 'hv372', 'hvq': 'hvq372'}[c[0]]}-{c[1] or 'default'}"
                                                    for c in SCORE_CASES])
 def test_scoring_builds_agree(cuda_lib, monkeypatch, case):
     key, threads, want = case
     ref_info, ref = _score_reference(key)
-    default = SCORE_CASES[0][2] if key == MV else SCORE_CASES[4][2]
+    default = next(want for k, threads, want in SCORE_CASES if k == key and threads is None)
     assert ref_info["score_threads_per_env"] == default, ref_info
     eng = _engine(key, monkeypatch, {"OPFG_SCORE_THREADS": threads} if threads else {})
     assert eng.info["score_threads_per_env"] == want, eng.info
