@@ -345,6 +345,7 @@ void opfg_row_program_destroy(OpfgRowProgram* program);
 /* Run the program on a subset of the table's rows only (host array of row numbers): rows whose stores
  * no kernel table ever reads need not be computed (row-level pruning by the table compiler). */
 int  opfg_row_program_select_rows(OpfgRowProgram* program, int32_t n_selected, const int32_t* rows /* host */);
+/* Fails, launching nothing, if a state cell the program touches on one of its rows is >= n_state. */
 int  opfg_row_program_run(const OpfgRowProgram* program, int64_t n_env, double* state, int32_t n_state,
                           void* cuda_stream);
 

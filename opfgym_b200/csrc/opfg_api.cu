@@ -206,6 +206,8 @@ struct OpfgGrid {
 struct OpfgRowProgram {
     int n_rows = 0, n_ops = 0, n_regs = 1;
     int n_items = 0;                 // rows the program runs on (all of them, or the selected subset)
+    int max_a = -1;                  // largest column start of a LOAD_STATE / STORE_STATE (-1: none)
+    int max_cell = -1;               // largest state cell the program touches on its items
     int32_t* rows = nullptr;         // device, [n_items] table row of every item; null = item i is row i
     std::vector<int> host_rows;
     OpfgRowOp* ops = nullptr;        // device
@@ -2085,11 +2087,15 @@ int opfg_row_program_create(int32_t n_rows, int32_t n_ops, const OpfgRowOp* ops,
         if (o.op >= OPFG_OP_ADD && o.op != OPFG_OP_STORE_STATE && (o.a < 0 || o.a >= 16)) return fail("row program: bad operand");
         if (o.op == OPFG_OP_STORE_STATE && (o.b < 0 || o.b >= 16)) return fail("row program: bad store register");
         if (o.op == OPFG_OP_LOAD_STATIC && (o.a < 0 || o.a + n_rows > n_static)) return fail("row program: static out of range");
+        if ((o.op == OPFG_OP_LOAD_STATE || o.op == OPFG_OP_STORE_STATE) && o.a < 0) return fail("row program: negative state cell");
     }
     auto* P = new OpfgRowProgram();
     P->n_rows = n_rows; P->n_ops = n_ops; P->n_items = n_rows;
-    for (int i = 0; i < n_ops; ++i)
+    for (int i = 0; i < n_ops; ++i) {
         if (ops[i].op != OPFG_OP_STORE_STATE) P->n_regs = std::max(P->n_regs, ops[i].dst + 1);
+        if (ops[i].op == OPFG_OP_LOAD_STATE || ops[i].op == OPFG_OP_STORE_STATE) P->max_a = std::max(P->max_a, ops[i].a);
+    }
+    P->max_cell = P->max_a >= 0 && n_rows > 0 ? P->max_a + n_rows - 1 : -1;
     P->host_ops.assign(ops, ops + n_ops);
     P->host_statics.assign(statics, statics + n_static);
     P->ops = (OpfgRowOp*)dev_alloc(sizeof(OpfgRowOp) * n_ops);
@@ -2112,11 +2118,14 @@ int opfg_row_program_select_rows(OpfgRowProgram* P, int32_t n_sel, const int32_t
     dev_put(P->rows, rows, sizeof(int32_t) * n_sel);
     P->host_rows.assign(rows, rows + n_sel);
     P->n_items = n_sel;
+    const int max_row = n_sel > 0 ? *std::max_element(rows, rows + n_sel) : -1;
+    P->max_cell = P->max_a >= 0 && max_row >= 0 ? P->max_a + max_row : -1;
     return 0;
 }
 
 int opfg_row_program_run(const OpfgRowProgram* P, int64_t n_env, double* state, int32_t n_state, void* stream) {
     if (!P || !state || n_env < 0) return fail("bad argument");
+    if (P->max_cell >= n_state) return fail("row program touches cell %d of a %d-cell state row", P->max_cell, n_state);
     if (n_env == 0 || P->n_items == 0) return 0;
 #ifdef OPFG_HOSTSIM
     (void)stream;
@@ -2219,11 +2228,17 @@ int opfg_reset_episode(const OpfgGrid* G, const OpfgBatch* B, const OpfgResetPla
                   host_regs, 1, seed, first_env, stream_base, random_action, action_stream_offset);
 #else
     const int n_in = G->d.n_inputs;
-    if (P->for_inputs != n_in) {      // does one reset write every input cell?  (then the row needs no copy-in)
-        std::vector<char> hit(std::max(n_in, 1), 0);
-        for (const auto& w : P->writes) for (int c : w) if (c < n_in) hit[c] = 1;
+    if (P->for_inputs != n_in) {
+        // The row needs no copy-in if every input cell is written before anything reads it: the first stage that
+        // touches a cell must write it and not read it (a stage that does both may read first, as in a += 1)
+        enum : char { UNTOUCHED, WRITTEN_FIRST, READ_FIRST };
+        std::vector<char> first(std::max(n_in, 1), UNTOUCHED);
+        for (size_t k = 0; k < P->host.size(); ++k) {
+            for (int c : P->reads[k]) if (c < n_in && first[c] == UNTOUCHED) first[c] = READ_FIRST;
+            for (int c : P->writes[k]) if (c < n_in && first[c] == UNTOUCHED) first[c] = WRITTEN_FIRST;
+        }
         bool all = true;
-        for (int c = 0; c < n_in && all; ++c) all = hit[c];
+        for (int c = 0; c < n_in && all; ++c) all = first[c] == WRITTEN_FIRST;
         P->covers_all = all; P->for_inputs = n_in;
     }
     // the row lives in shared memory if everything the reset touches lies in the input part

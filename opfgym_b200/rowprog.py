@@ -26,10 +26,11 @@ N_REG = 16
 
 
 class Expr:
-    __slots__ = ("op", "args", "imm", "start")
+    __slots__ = ("op", "args", "imm", "start", "seq")
 
-    def __init__(self, op, args=(), imm=0.0, start=0):
-        self.op, self.args, self.imm, self.start = op, tuple(args), float(imm), int(start)
+    def __init__(self, op, args=(), imm=0.0, start=0, seq=0):
+        # seq (LOAD_STATE): stores made before the handle -- it reads the column as it was then
+        self.op, self.args, self.imm, self.start, self.seq = op, tuple(args), float(imm), int(start), int(seq)
 
     @staticmethod
     def wrap(v):
@@ -73,7 +74,8 @@ class RowProgram:
         if column not in self._cols:
             lay = self.env.program.layout
             if lay.has(self.table, column):
-                self._cols[column] = Expr(LOAD_STATE, start=lay.columns[(self.table, column)][0])
+                self._cols[column] = Expr(LOAD_STATE, start=lay.columns[(self.table, column)][0],
+                                          seq=len(self.stores))
             else:
                 if column not in self._static_index:
                     self._static_index[column] = len(self.statics) * self.n_rows
@@ -115,15 +117,14 @@ class RowProgram:
             if sig:
                 groups.setdefault(sig, []).append(r)
         out = []
-        all_stores = self.stores
         for sig, rows in groups.items():
-            self.stores = [all_stores[i] for i in sig]
-            ops, statics = self.compile()
+            ops, statics = self.compile(sig)
             out.append((None if len(rows) == self.n_rows else np.asarray(rows, np.int32), ops, statics))
-        self.stores = all_stores
         return out
 
-    def compile(self):
+    def compile(self, keep=None):
+        """Register program of the stores ``keep`` (indices into ``self.stores``; default all of them)."""
+        stores = [(i, *self.stores[i]) for i in (range(len(self.stores)) if keep is None else keep)]
         uses: dict[int, int] = {}
 
         def count(e):
@@ -131,8 +132,21 @@ class RowProgram:
             if uses[id(e)] == 1:
                 for a in e.args:
                     count(a)
-        for _, e in self.stores:
+        for _, _, e in stores:
             count(e)
+        # LOAD_STATE handles per column, with the last store that reads each of them
+        loads_of: dict[int, dict[int, tuple]] = {}
+
+        def find_loads(e, i, seen):
+            if id(e) in seen:
+                return
+            seen.add(id(e))
+            if e.op == LOAD_STATE:
+                loads_of.setdefault(e.start, {})[id(e)] = (e, i)
+            for a in e.args:
+                find_loads(a, i, seen)
+        for i, _, e in stores:
+            find_loads(e, i, set())
         ops, reg_of, free = [], {}, list(range(N_REG - 1, -1, -1))
 
         def release(e):
@@ -157,7 +171,11 @@ class RowProgram:
             else:
                 ops.append((e.op, dst, regs[0], regs[1] if len(regs) > 1 else 0, 0.0))
             return dst
-        for start, e in self.stores:
+        for i, start, e in stores:
+            # a handle taken before this store still reads the old value: load it now if a later store uses it
+            for h, last in loads_of.get(start, {}).values():
+                if h.seq <= i < last and id(h) not in reg_of and uses[id(h)] > 0:
+                    emit(h)
             r = emit(e)
             ops.append((STORE_STATE, 0, start, r, 0.0))
             release(e)

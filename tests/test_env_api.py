@@ -7,6 +7,7 @@ import torch
 from opfgym_b200 import envs
 from opfgym_b200 import reward as R
 from opfgym_b200.data_split import define_test_train_split
+from opfgym_b200.engine import Engine
 from tests.hostsim.harness import TorchHostSimEngine
 
 KW = dict(engine_cls=TorchHostSimEngine, n_profile_steps=672, obs_dtype="float64")
@@ -338,22 +339,34 @@ def test_step_host_matches_step():
     np.testing.assert_array_equal(r_host, r_dev.numpy())
 
 
-@pytest.mark.parametrize("cls_name,kw", [("VoltageControl", {}), ("LoadShedding", {}),
-                                         ("EcoDispatch", {"initial_action": "random"}),
-                                         ("MaxRenewable", {})])
-def test_fused_reset_equals_kernel_sequence(cls_name, kw):
+FUSED_RESET_ENVS = [("VoltageControl", {}), ("LoadShedding", {}), ("EcoDispatch", {"initial_action": "random"}),
+                    ("MaxRenewable", {}), ("QMarket", {}), ("LoadSheddingReconfiguration", {})]
+FUSED_RESET_CASES = \
+    [pytest.param(name, kw, 4, "host", id=f"{name}-kw{k}") for k, (name, kw) in enumerate(FUSED_RESET_ENVS)] + \
+    [pytest.param(name, kw, n, "host", id=f"{name}-n{n}") for name, kw in FUSED_RESET_ENVS[:3] for n in (1, 129)] + \
+    [pytest.param(name, kw, n, "cuda", id=f"{name}-n{n}-cuda", marks=pytest.mark.gpu)
+     for name, kw in FUSED_RESET_ENVS for n in (1, 4, 129)]
+
+
+@pytest.mark.parametrize("cls_name,kw,n,engine", FUSED_RESET_CASES)
+def test_fused_reset_equals_kernel_sequence(request, cls_name, kw, n, engine):
     """opfg_reset_episode (one launch) vs the recorded sequence sampler / hook programs / initial
-    action / set-points / observe: bit-identical state rows and observations, episode after episode."""
+    action / set-points / observe: bit-identical state rows and observations, episode after episode.
+    On CUDA the fused reset runs one 128-thread CTA per environment with the row in shared memory,
+    where a wrong stage grouping is a race; the sequence is the separate CUDA kernels."""
     cls = getattr(envs, cls_name)
-    fused = make(cls, n=4, **kw)                     # automatic for the built-in envs at small batch sizes
-    plain = make(cls, n=4, fused_reset=False, **kw)
+    if engine == "cuda":
+        request.getfixturevalue("cuda_lib")
+        kw = dict(kw, engine_cls=Engine, prefetch_reset=False)
+    fused = make(cls, n=n, **kw)                     # automatic for the built-in envs at small batch sizes
+    plain = make(cls, n=n, fused_reset=False, **kw)
     assert fused.fused_reset and not plain.fused_reset
     of, _ = fused.reset(seed=31)          # recorded
     op, _ = plain.reset(seed=31)
     assert torch.equal(of, op)
     n_act = fused.single_action_space.shape[0]
     for k in range(3):
-        act = torch.rand(4, n_act, dtype=torch.float64, generator=torch.Generator().manual_seed(k))
+        act = torch.rand(n, n_act, dtype=torch.float64, generator=torch.Generator().manual_seed(k)).to(fused.device)
         rf, rp = fused.step(act), plain.step(act)      # auto-reset: replayed by the fused kernel
         assert fused._reset_plans and not plain._reset_plans
         assert torch.equal(rf[0], rp[0]) and torch.equal(rf[1], rp[1])
