@@ -83,7 +83,8 @@ typedef struct {
     int32_t init_dc;        /* 1: DC-power-flow angle start (pandapower init='dc')        */
     int32_t enforce_q_lims; /* 1: PV->PQ outer loop of pandapower's enforce_q_lims        */
     int32_t threads_per_env;/* 0 = choose from grid size (32/64/128)                      */
-    int32_t ordering;       /* 0 = auto, 1 = min-degree, 2 = independent-set, 3 = least fill work      */
+    int32_t ordering;       /* 0 = auto, 1 = min-degree, 2 = independent-set, 3 = least fill work;
+                               auto roots each tree of a radial grid at its centre (fewest levels)   */
     int32_t pf_kernel;      /* 0 = auto, 1 = one CTA per environment (level-scheduled block LU in shared
                                memory), 2 = one LANE per environment (row-wise LU, Jacobian never stored,
                                state in global scratch), 3 = fused kernel for radial grids (8-32 lanes per

@@ -805,9 +805,11 @@ static GridDev staged_view(const GridDev& d, int stage) {
 #endif
 
 // lanes per environment of the fused radial kernel (also the cap of its balanced levels).  Measured on
-// the 122-bus grid (B200, 32 768 environments): 8 lanes 1.27 ms, 16 lanes 1.00 ms, 32 lanes 1.26 ms --
-// the kernel is bound by the latency of its level chain, more lanes mean fewer rounds per level until
-// the idle lanes of the narrow levels cost more issue slots than the rounds save.
+// the 122-bus grid with the centre-rooted order (B200 at 1000 W, 32 768 environments, opfg_pf_solve incl.
+// the DC-start GEMM): 8 lanes 1.051 ms (17 levels), 16 lanes 0.758 ms (14 levels), 32 lanes 0.990 ms
+// (14 levels, 16 environments per SM) -- the kernel is bound by the latency of its level chain, more lanes
+// mean fewer rounds per level until the idle lanes of the narrow levels cost more issue slots than the
+// rounds save.
 constexpr int TREE_LANES = 16;
 
 // Radial grid with the dense DC pre-pass: the fused kernel (pf_kernel 0 = auto or 3 = radial)
@@ -917,15 +919,12 @@ int opfg_grid_create(const OpfgGridDesc* desc, OpfgGrid** out) {
         const int pf_kernel = desc->pf_kernel;
         G->pf_kernel = pf_kernel;
         const bool want_lanes = pf_kernel == 2;     // measured slower than the CTA kernels on B200 (DESIGN.md): opt-in
-        analyse(nb, type, active, (desc->ordering == 0 && want_lanes) ? 3 : desc->ordering, T > 0 ? T : 32, s);
-        if (desc->ordering == 0 && pf_kernel != 1 && pf_kernel != 2 && s.fill_ids.size() > 0) {
-            // a radial grid has a fill-free (leaf-first) order, which is what the fused kernel needs
-            Symbolic leaf_first;
-            analyse(nb, type, active, 1, T > 0 ? T : 32, leaf_first, TREE_LANES);
-            bool forest = leaf_first.fill_ids.empty();
-            for (int k = 0; k < leaf_first.n && forest; ++k) forest = leaf_first.up_ptr[k + 1] - leaf_first.up_ptr[k] <= 1;
-            if (forest) s = leaf_first;
-        }
+        if (desc->ordering < 0 || desc->ordering > 3) { delete G; return fail("unknown ordering %d", desc->ordering); }
+        // a radial grid has a fill-free (leaf-first) order, which is what the fused kernel needs; rooting every
+        // tree at its centre makes its level chain the shortest such an order has
+        const bool centre_rooted = desc->ordering == 0 && pf_kernel != 1 && pf_kernel != 2 && is_forest(nb, type, active);
+        const int ordering = centre_rooted ? 4 : ((desc->ordering == 0 && want_lanes) ? 3 : desc->ordering);
+        analyse(nb, type, active, ordering, T > 0 ? T : 32, s, centre_rooted ? TREE_LANES : 0);
         if (T <= 0) T = s.n_blocks <= 1000 ? 64 : 128;   // measured: 64 on the MV grids (~450 blocks), 128 on HV (~1900)
         for (size_t c = 0; c < s.yc_branch.size(); ++c)
             if (s.yc_role[c] != 4) s.yc_branch[c] = active_row[s.yc_branch[c]];
@@ -1857,8 +1856,9 @@ int opfg_pf_solve(const OpfgGrid* G, const OpfgBatch* B, void* stream) {
         const bool dyn = G->d.n_dyn > 0 && B->yval;
         constexpr int T = TREE_LANES;
         // at most 24 environments take the register cap of 384 threads (155 instead of 128 registers).  Measured on
-        // B200 (122-bus grid, 32 768 environments): 0.80 instead of 0.90 ms -- under the 128-register cap the
-        // staged-table base addresses were recomputed at their use sites
+        // B200 (122-bus grid, 32 768 environments, the 18-level minimum-degree order): 0.80 instead of 0.90 ms --
+        // under the 128-register cap the staged-table base addresses were recomputed at their use sites.  The
+        // 14-level centre-rooted order changes neither the registers nor the environments per SM
         void (*fns[4])(GridDev, OpfgBatch, int, int) = {k_pf_tree<T, false, 512>, k_pf_tree<T, true, 512>,
                                                         k_pf_tree<T, false, 384>, k_pf_tree<T, true, 384>};
         if (!Gm->tree_attr_set) {      // per grid, hence per device

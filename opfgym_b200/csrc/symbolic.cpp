@@ -193,33 +193,126 @@ Order make_order(const std::vector<std::set<int>>& adj0, const std::vector<int>&
     return o;
 }
 
+// Breadth-first distances from `root` (-1 outside its component); returns the nodes in visiting order.
+std::vector<int> bfs(const std::vector<std::set<int>>& adj, int root, std::vector<int>& dist,
+                     std::vector<int>* from = nullptr) {
+    dist.assign(adj.size(), -1);
+    if (from) from->assign(adj.size(), -1);
+    std::vector<int> seen{root};
+    dist[root] = 0;
+    for (size_t i = 0; i < seen.size(); ++i)
+        for (int a : adj[seen[i]])
+            if (dist[a] < 0) {
+                dist[a] = dist[seen[i]] + 1;
+                if (from) (*from)[a] = seen[i];
+                seen.push_back(a);
+            }
+    return seen;
+}
+
+// Leaf-first order of a forest with every tree rooted at a centre (the middle of a longest path, found by
+// two BFS passes): nodes by decreasing depth from their tree's centre.  Eliminating a node removes a leaf
+// of what is left, so there is no fill and each pivot keeps one later neighbour (its parent), and the
+// dependency chain of a tree is its radius + 1 levels: the fewest any fill-free order has, since a
+// leaf-first order is a rooted tree and no root gives a lower height.  A tree with two centres takes the
+// one that gives fewer levels under `level_cap`, then the lower node id.
+std::vector<int> centre_rooted_sequence(const std::vector<std::set<int>>& adj, int threads, int level_cap) {
+    const int n = (int)adj.size();
+    std::vector<int> comp_of(n, -1), dist, from;
+    std::vector<std::array<int, 2>> centres;                 // per component; [1] = -1 with one centre
+    for (int v0 = 0; v0 < n; ++v0) {
+        if (comp_of[v0] >= 0) continue;
+        const int u = bfs(adj, v0, dist).back();             // farthest from v0: one end of a longest path
+        const std::vector<int> seen = bfs(adj, u, dist, &from);
+        std::vector<int> path{seen.back()};                  // the other end, walked back to u
+        while (path.back() != u) path.push_back(from[path.back()]);
+        const int len = (int)path.size() - 1;
+        for (int v : seen) comp_of[v] = (int)centres.size();
+        std::array<int, 2> c{path[len / 2], len % 2 ? path[len / 2 + 1] : -1};
+        if (c[1] >= 0 && c[1] < c[0]) std::swap(c[0], c[1]);
+        centres.push_back(c);
+    }
+    std::vector<int> root(centres.size());
+    for (size_t c = 0; c < centres.size(); ++c) root[c] = centres[c][0];
+    auto sequence = [&]() {
+        std::vector<int> depth(n);
+        for (size_t c = 0; c < centres.size(); ++c) {
+            bfs(adj, root[c], dist);
+            for (int v = 0; v < n; ++v) if (comp_of[v] == (int)c) depth[v] = dist[v];
+        }
+        std::vector<int> seq(n);
+        for (int v = 0; v < n; ++v) seq[v] = v;
+        std::stable_sort(seq.begin(), seq.end(), [&](int a, int b) { return depth[a] > depth[b]; });
+        return seq;
+    };
+    if (level_cap > 0) {
+        auto levels = [&]() { return (int)make_order(adj, sequence(), threads, "", level_cap).level_ptr.size() - 1; };
+        int best = levels();
+        for (size_t c = 0; c < centres.size(); ++c) {
+            if (centres[c][1] < 0) continue;
+            root[c] = centres[c][1];
+            const int other = levels();
+            if (other < best) best = other;
+            else root[c] = centres[c][0];
+        }
+    }
+    return sequence();
+}
+
 inline int64_t key(int i, int j) { return ((int64_t)i << 32) | (uint32_t)j; }
 
-}  // namespace
-
-void analyse(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches,
-             int ordering, int threads, Symbolic& s, int level_cap) {
-    s = Symbolic();
-    s.nb = nb;
-    std::vector<int> node_of_bus(nb, -1), bus_of_node;
+// graph of the non-reference buses (self loops dropped, parallel branches collapse); bus_of_node: the bus of each node
+std::vector<std::set<int>> bus_graph(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches,
+                                     std::vector<int>& bus_of_node) {
+    std::vector<int> node_of_bus(nb, -1);
+    bus_of_node.clear();
     for (int b = 0; b < nb; ++b)
         if (bus_type[b] != 3) { node_of_bus[b] = (int)bus_of_node.size(); bus_of_node.push_back(b); }
-    const int n = (int)bus_of_node.size();
-    s.n = n;
-    std::vector<std::set<int>> adj(n);
+    std::vector<std::set<int>> adj(bus_of_node.size());
     for (const auto& br : branches) {
         if (br.f == br.t) continue;
         int a = node_of_bus[br.f], b = node_of_bus[br.t];
         if (a >= 0 && b >= 0) { adj[a].insert(b); adj[b].insert(a); }
     }
+    return adj;
+}
+
+}  // namespace
+
+bool is_forest(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches) {
+    std::vector<int> bus_of_node, dist;
+    const auto adj = bus_graph(nb, bus_type, branches, bus_of_node);
+    const int n = (int)adj.size();
+    size_t edges = 0;
+    for (const auto& a : adj) edges += a.size();
+    edges /= 2;
+    int components = 0;
+    std::vector<char> seen(n, 0);
+    for (int v = 0; v < n; ++v) {
+        if (seen[v]) continue;
+        ++components;
+        for (int u : bfs(adj, v, dist)) seen[u] = 1;
+    }
+    return edges == (size_t)(n - components);
+}
+
+void analyse(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches,
+             int ordering, int threads, Symbolic& s, int level_cap) {
+    s = Symbolic();
+    s.nb = nb;
+    std::vector<int> bus_of_node;
+    const std::vector<std::set<int>> adj = bus_graph(nb, bus_type, branches, bus_of_node);
+    const int n = (int)bus_of_node.size();
+    s.n = n;
     std::vector<Order> cands;
     const bool least_work = ordering == 3;     // lane-per-environment kernel: levels are irrelevant, fill is work
     if (least_work) ordering = 0;
-    if (ordering == 0 || ordering == 1) cands.push_back(make_order(adj, min_degree_sequence(adj), threads, "min_degree", level_cap));
+    if (ordering == 0 || ordering == 1) cands.push_back(make_order(adj, min_degree_sequence(adj), threads, "min_degree"));
     if (ordering == 0 || ordering == 2) {
         cands.push_back(make_order(adj, independent_set_sequence(adj, 0), threads, "independent_set"));
         cands.push_back(make_order(adj, independent_set_sequence(adj, 1), threads, "independent_set+1"));
     }
+    if (ordering == 4) cands.push_back(make_order(adj, centre_rooted_sequence(adj, threads, level_cap), threads, "centre_rooted", level_cap));
     if (cands.empty()) throw std::runtime_error("unknown ordering");
     const Order* best = &cands[0];
     auto work = [](const Order& o) {           // Schur-update pairs: sum over pivots of |struct|^2

@@ -70,9 +70,14 @@ struct LaneSchedule {
 };
 void build_lane_schedule(const Symbolic& s, LaneSchedule& out);
 
+// true when the graph of the non-reference buses (self loops and parallel branches dropped) is a forest:
+// edges == nodes - components
+bool is_forest(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches);
+
 // ordering: 0 auto (cheapest by the CTA kernel's cost model), 1 minimum degree, 2 independent-set rounds,
-// 3 least work (fewest Schur-update pairs; what the lane-per-environment kernel wants)
-// level_cap > 0 (minimum-degree order only): at most that many pivots per level (balanced levels)
+// 3 least work (fewest Schur-update pairs; what the lane-per-environment kernel wants), 4 leaf-first with
+// every tree rooted at its centre (forests only: no fill, radius + 1 levels per tree; the radial kernel's order)
+// level_cap > 0 (centre-rooted order only): at most that many pivots per level (balanced levels)
 void analyse(int nb, const std::vector<int>& bus_type, const std::vector<BranchHost>& branches,
              int ordering, int threads_per_env, Symbolic& out, int level_cap = 0);
 
